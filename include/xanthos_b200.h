@@ -243,6 +243,28 @@ int xan_agg_to_year(const double *d_src, double *d_dst, int ncell, int nmonths, 
 /* basin aggregate: out[m][b] = nansum_{c in basin b} src[m][c] * w[c] (w may be NULL = 1) */
 int xan_basin_sum(const xan_abcd_plan *plan, const double *d_src, const double *d_w,
                   int nmonths, int ld, double *d_out, void *stream);
+/* mm -> km3 (out_writer.py:114-115): dst[t][c] = src[t][c] * scale[c] over [ntime][ld]; d_dst may be d_src */
+int xan_scale_cells(const double *d_src, const double *d_scale, int ncell, int ntime, int ld,
+                    double *d_dst, void *stream);
+
+/* ---- across-member statistics of an ensemble (csrc/ensemble_stats.cu) ------------------------- */
+/* State per (time, cell), month-major [ntime][ld], 16-byte aligned: d_sm = (sum, m2) and d_mm = (min, max) as
+ * interleaved pairs of doubles ([ntime][ld][2] each).  Operations are + - * / sqrt only (no FMA contraction), so the
+ * results are bitwise those of oracle/ensemble_stats.py.
+ *   xan_ens_stats_update    adds member number n (1-based, member order) with values d_x [ntime][ld]: n == 1
+ *                           initialises (sum = x, m2 = 0, min = max = x); later members add x to the sequential sum
+ *                           (numpy.mean(stack, axis=0) = sum / n bitwise), update m2 by Welford with the running mean
+ *                           sum / n, and min / max propagate NaN like numpy.min / numpy.max.
+ *   xan_ens_stats_merge     Chan et al.: partial a of na members absorbs partial b of nb members in place:
+ *                           sum = sa + sb, m2 = m2a + m2b + d * d * na * nb / (na + nb) with d = sb / nb - sa / na.
+ *   xan_ens_stats_finalize  numpy.mean, numpy.std(ddof) = sqrt(m2 / (n - ddof)), numpy.min, numpy.max over the n
+ *                           members, written cell-major [ncell][ntime]; any output may be NULL. */
+int xan_ens_stats_update(const double *d_x, double *d_sm, double *d_mm, int ncell, int ntime, int ld, int n,
+                         void *stream);
+int xan_ens_stats_merge(double *d_sm_a, double *d_mm_a, const double *d_sm_b, const double *d_mm_b, int ncell,
+                        int ntime, int ld, int na, int nb, void *stream);
+int xan_ens_stats_finalize(const double *d_sm, const double *d_mm, int ncell, int ntime, int ld, int n, int ddof,
+                           double *d_mean, double *d_std, double *d_min, double *d_max, void *stream);
 
 /* ---- post-processing scans on the resident fields (SURVEY.md section 8 row f3) -------------- */
 /* DroughtStats.droughtstats (xanthos/drought/drought_stats.py:85-148): d_hydro [nmonths][ld],

@@ -79,6 +79,10 @@ SIGNATURES = {
     'xan_drought_thresholds': (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_double, _P, c_int, _P]),
     'xan_group_sum': (c_int, [_P, _P, _P, c_int, c_int, c_int, _P, _P]),
     'xan_year_sum_scaled': (c_int, [_P, _P, c_int, c_int, c_int, _P, _P]),
+    'xan_scale_cells': (c_int, [_P, _P, c_int, c_int, c_int, _P, _P]),
+    'xan_ens_stats_update': (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, _P]),
+    'xan_ens_stats_merge': (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, _P]),
+    'xan_ens_stats_finalize': (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P]),
     'xan_de_init': (c_int, [_P, c_int, c_int, c_int, ctypes.c_ulonglong, _P]),
     'xan_de_trial': (c_int, [_P, _P, _P, c_int, c_int, c_int, c_int, _P, _P, ctypes.c_ulonglong, c_int, c_double,
                              c_double, c_double, _P, _P, _P]),
@@ -93,6 +97,7 @@ KERNELS_PER_CALL = {
     'xan_thornthwaite_daylight': 1, 'xan_pm_pet': 1, 'xan_abcd_run': 3, 'xan_abcd_kge_batch': 1,
     'xan_mrtm_route': 1, 'xan_mrtm_route_batch': 1, 'xan_hargreaves_pet': 1, 'xan_gwam_run': 1, 'xan_agg_to_year': 1, 'xan_basin_sum': 1,
     'xan_drought_stats': 1, 'xan_drought_thresholds': 1, 'xan_group_sum': 1, 'xan_year_sum_scaled': 1,
+    'xan_scale_cells': 1, 'xan_ens_stats_update': 1, 'xan_ens_stats_merge': 1, 'xan_ens_stats_finalize': 1,
     'xan_de_init': 1, 'xan_de_trial': 1, 'xan_de_select': 1,
 }
 launch_count = 0

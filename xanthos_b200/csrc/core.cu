@@ -106,6 +106,15 @@ __global__ void agg_to_year_kernel(const double *__restrict__ src, double *__res
     dst[(size_t)y * ld + c] = acc;
 }
 
+// OutWriter's mm -> km3 conversion (out_writer.py:114-115): every time row times a per-cell factor (src may be dst)
+__global__ void scale_cells_kernel(const double *src, const double *__restrict__ scale, int ncell, int ld,
+                                   double *dst) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= ncell) return;
+    const size_t i = (size_t)blockIdx.y * ld + c;
+    dst[i] = src[i] * scale[c];
+}
+
 }  // namespace xan
 
 using namespace xan;
@@ -175,6 +184,17 @@ int xan_agg_to_year(const double *d_src, double *d_dst, int ncell, int nmonths, 
     dim3 grid(ceil_div(ncell, 256), nmonths / 12);
     agg_to_year_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_src, d_dst, ncell, nmonths / 12, ld,
                                                               take_mean);
+    XAN_CUDA_CHECK(cudaGetLastError());
+    return XAN_OK;
+}
+
+int xan_scale_cells(const double *d_src, const double *d_scale, int ncell, int ntime, int ld, double *d_dst,
+                    void *stream) {
+    XAN_REQUIRE(d_src && d_scale && d_dst, "xan_scale_cells: null pointer");
+    XAN_REQUIRE(ncell > 0 && ntime > 0 && ntime <= 65535 && ld >= ncell, "xan_scale_cells: bad shape %d x %d (ld %d)",
+                ncell, ntime, ld);
+    dim3 grid(ceil_div(ncell, 256), ntime);
+    scale_cells_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_src, d_scale, ncell, ld, d_dst);
     XAN_CUDA_CHECK(cudaGetLastError());
     return XAN_OK;
 }

@@ -20,6 +20,10 @@ fixed ring of device staging buffers (no allocation inside the pipeline).  Only 
 keeps PET, AET, Q, Sav, ChStorage and Avg_ChFlow of a scenario in host memory but writes `output_vars` only,
 data_writer/out_writer.py:60-110).  With torch.distributed initialised the members are dealt in contiguous blocks to the ranks
 (no collective in the data path) and the basin aggregates [n_members, 2, nmonths, n_basins] are gathered at the end.
+
+An `OutputSpec` applies the reference's output options (yearly, km3, basin / country / region sums) and across-member
+statistics on the device, in front of the copy back (`run_ensemble(..., spec=...)`): the copy back, not the compute, is
+what limits multi-GPU runs, and a user who wants reduced output no longer pulls every monthly grid to the host.
 """
 
 from types import SimpleNamespace
@@ -35,6 +39,57 @@ from .routing import mrtm as mrtm_mod
 PM_FORCING = ('tair_load', 'TMIN_load', 'rhs_load', 'wind_load', 'rsds_load', 'rlds_load')
 FORCING = PM_FORCING + ('precip', 'tmin')
 OUTPUTS = ('pet', 'aet', 'q', 'soilmoisture', 'chstorage', 'avgchflow')
+GROUP_SCALES = ('basin', 'country', 'region')
+STATS = ('mean', 'std', 'min', 'max')
+
+
+class OutputSpec:
+    """
+    What the ensemble runner computes from each member's monthly outputs on the device before anything is copied back:
+
+      output_in_year  yearly sum (mean for avgchflow) of every variable, NaN skipped (OutWriter.write, out_writer.py:103-112)
+      output_unit     'mm' or 'km3': mm -> km3 by `area / 1e6` after the yearly aggregation, never for avgchflow
+                      (out_writer.py:114-115)
+      group_sums      subset of ('basin', 'country', 'region'): sums of q after its conversion over the cells of every
+                      id > 0, in cell-index order, NaN skipped, [max(ids), ntime] (OutWriter.write_aggregates,
+                      out_writer.py:250-265)
+      member_fields   False: no per-member grid is copied back (group sums and statistics only)
+      stats           subset of ('mean', 'std', 'min', 'max') over the members, per (cell, time step) of every output
+                      variable; std with `ddof` like numpy.std
+
+    Every member's grids and group sums are bit-identical to what OutWriter.write / write_aggregates produce from that
+    member's monthly outputs.  chstorage is never written through OutWriter: it is rejected with yearly or km3 output.
+    """
+
+    def __init__(self, output_in_year=False, output_unit='mm', group_sums=(), member_fields=True, stats=(), ddof=0):
+        if output_unit not in ('mm', 'km3'):
+            raise C.ValidationException("output_unit must be 'mm' or 'km3', not {!r}".format(output_unit))
+        group_sums, stats = tuple(group_sums), tuple(stats)
+        bad = [g for g in group_sums if g not in GROUP_SCALES] + [s for s in stats if s not in STATS]
+        if bad or len(set(group_sums)) != len(group_sums) or len(set(stats)) != len(stats):
+            raise C.ValidationException("unknown or repeated group sums / statistics {} (choose from {} and {})".format(
+                list(group_sums) + list(stats), GROUP_SCALES, STATS))
+        if int(ddof) != ddof or ddof < 0:
+            raise C.ValidationException("ddof must be a non-negative integer, not {!r}".format(ddof))
+        self.output_in_year, self.output_unit = bool(output_in_year), output_unit
+        self.group_sums, self.member_fields, self.stats, self.ddof = group_sums, bool(member_fields), stats, int(ddof)
+
+    @classmethod
+    def from_settings(cls, settings, member_fields=True, stats=(), ddof=0):
+        """The output options of a parsed configuration (data_reader.ini_reader.ConfigReader): OutputInYear,
+        OutputUnit and the AggregateRunoffBasin / Country / GCAMRegion flags."""
+        unit = int(settings.OutputUnit)
+        if unit not in (0, 1):
+            raise C.ValidationException("OutputUnit must be 0 (mm) or 1 (km3), not {}".format(unit))
+        flags = (settings.AggregateRunoffBasin, settings.AggregateRunoffCountry, settings.AggregateRunoffGCAMRegion)
+        return cls(output_in_year=bool(int(settings.OutputInYear)), output_unit=('mm', 'km3')[unit],
+                   group_sums=tuple(g for g, f in zip(GROUP_SCALES, flags) if int(f)), member_fields=member_fields,
+                   stats=stats, ddof=ddof)
+
+    def __repr__(self):
+        return ('OutputSpec(output_in_year={}, output_unit={!r}, group_sums={}, member_fields={}, stats={}, ddof={})'
+                .format(self.output_in_year, self.output_unit, self.group_sums, self.member_fields, self.stats,
+                        self.ddof))
 
 
 def lossless_float32(member, pin=True):
@@ -66,7 +121,7 @@ class EnsembleStatics:
 
     def __init__(self, ncell, start_yr, end_yr, pm_tables, lct_load, elev, water_idx, snow_idx, lc_years, nlcs,
                  n_basins, basin_ids, abcd_pars, area, flow_dist, velocity, upstream_matrix, ndays, dt=3 * 3600,
-                 runoff_spinup=None, routing_spinup=None):
+                 runoff_spinup=None, routing_spinup=None, country_ids=None, region_ids=None):
         torch = C.torch_cuda()
         self.ncell, self.start_yr, self.end_yr = int(ncell), int(start_yr), int(end_yr)
         self.nmonths = (self.end_yr - self.start_yr + 1) * 12
@@ -87,6 +142,34 @@ class EnsembleStatics:
         self.dt = float(dt)
         self.runoff_spinup = self.nmonths if runoff_spinup is None else int(runoff_spinup)
         self.routing_spinup = self.nmonths if routing_spinup is None else int(routing_spinup)
+        self.area = area
+        self.group_ids = {'basin': self.basin_ids, 'country': country_ids, 'region': region_ids}
+        self._group_tables, self._km3 = {}, None
+
+    def group_table(self, scale):
+        """Device (order, offsets, ngroups) of xan_group_sum for 'basin' / 'country' / 'region', built once."""
+        hit = self._group_tables.get(scale)
+        if hit is None:
+            from .diagnostics.time_series import group_plan
+            ids = self.group_ids.get(scale)
+            if ids is None:
+                raise C.ValidationException("{} group sums requested, but no {}_ids were given to EnsembleStatics".format(
+                    scale, scale))
+            ids = np.asarray(ids).astype(np.int64).reshape(-1)
+            if ids.shape[0] != self.ncell:
+                raise C.ValidationException("{}_ids has {} entries for {} cells".format(scale, ids.shape[0], self.ncell))
+            order, offsets, ng = group_plan(ids)
+            if ng < 1:
+                raise C.ValidationException("{}_ids has no positive id".format(scale))
+            torch = C.torch_cuda()
+            hit = self._group_tables[scale] = (torch.from_numpy(order).cuda(), torch.from_numpy(offsets).cuda(), ng)
+        return hit
+
+    def km3_scale(self):
+        """Device vector area / 1e6, OutWriter.conversion_mm_km3 (not d_area_km3 = area * 1e-6: the last bit differs)."""
+        if self._km3 is None:
+            self._km3 = C.dev_vector(np.asarray(self.area, dtype=np.float64).reshape(-1) / 1e6)
+        return self._km3
 
     def data_ns(self, fields):
         d = dict(self.tables)
@@ -97,7 +180,7 @@ class EnsembleStatics:
 
 
 class EnsembleRunner:
-    def __init__(self, statics, output_vars=('q', 'avgchflow'), aggregates=True, prefetch_depth=4, group=2):
+    def __init__(self, statics, output_vars=('q', 'avgchflow'), aggregates=True, prefetch_depth=4, group=2, spec=None):
         torch = C.torch_cuda()
         self.prefetch_depth = max(1, int(prefetch_depth))   # members whose forcing may be on its way ahead of the compute
         self.group = max(1, int(group))                     # members routed by one launch
@@ -105,6 +188,15 @@ class EnsembleRunner:
         if bad:
             raise C.ValidationException("unknown output variable(s) {}; choose from {}".format(bad, OUTPUTS))
         self.s, self.output_vars, self.aggregates = statics, tuple(output_vars), bool(aggregates)
+        self.spec = spec
+        self.ntime = statics.nmonths // 12 if spec is not None and spec.output_in_year else statics.nmonths
+        if spec is not None:
+            if 'chstorage' in self.output_vars and (spec.output_in_year or spec.output_unit == 'km3'):
+                raise C.ValidationException("chstorage has no yearly or km3 output (OutWriter never writes it)")
+            self._groups = {g: statics.group_table(g) for g in spec.group_sums}
+            # group sums are of q as it is written (after the yearly aggregation and the unit conversion)
+            self._reduce_vars = self.output_vars + (('q',) if spec.group_sums and 'q' not in self.output_vars else ())
+        self._stats_state, self.n_stats = None, 0   # across-member accumulators: var -> (sum, m2) and (min, max)
         # One pair of copy streams per process and device, not per runner: torch's caching allocator keeps freed blocks
         # per STREAM, so every new stream starts with an empty pool - a runner per run_ensemble call with fresh streams
         # left 6 - 9 GB of staging blocks cached under dead streams per call, and after a dozen calls the allocator had
@@ -237,10 +329,50 @@ class EnsembleRunner:
             results.append((out, agg))
         return results
 
+    def _reduce(self, out):
+        """The member's outputs as the spec asks for them (compute stream): yearly aggregation, km3, group sums of q,
+        and the member added to the across-member statistics.  Returns ({var: Field [ntime][ld]}, {scale: [ng, ntime]})."""
+        s, spec, lib = self.s, self.spec, C.lib()
+        red = {}
+        for v in self._reduce_vars:
+            f = out[v]
+            if spec.output_in_year:
+                y = C.Field.empty(s.ncell, self.ntime, f.ld)
+                C.check(lib.xan_agg_to_year(C.ptr(f.t), C.ptr(y.t), s.ncell, s.nmonths, f.ld, int(v == 'avgchflow'),
+                                            C.stream_ptr()))
+                f = y
+            if spec.output_unit == 'km3' and v != 'avgchflow':
+                dst = f if spec.output_in_year else C.Field.empty(s.ncell, self.ntime, f.ld)   # monthly: keep the original
+                C.check(lib.xan_scale_cells(C.ptr(f.t), C.ptr(s.km3_scale()), s.ncell, self.ntime, f.ld, C.ptr(dst.t),
+                                            C.stream_ptr()))
+                f = dst
+            red[v] = f
+        groups = {}
+        for g, (d_order, d_off, ng) in self._groups.items():
+            t = self._torch.empty((ng, self.ntime), dtype=self._torch.float64, device='cuda')
+            C.check(lib.xan_group_sum(C.ptr(red['q'].t), C.ptr(d_order), C.ptr(d_off), ng, self.ntime, red['q'].ld,
+                                      C.ptr(t), C.stream_ptr()))
+            groups[g] = t
+        if spec.stats:          # members arrive in order: the sequential sum is numpy's over the stacked members
+            self.n_stats += 1
+            for v in self.output_vars:
+                sm, mm = self._stats_state[v]
+                if red[v].ld != s.ld:
+                    raise RuntimeError("ensemble statistics: field pitch {} differs from {}".format(red[v].ld, s.ld))
+                C.check(lib.xan_ens_stats_update(C.ptr(red[v].t), C.ptr(sm), C.ptr(mm), s.ncell, self.ntime,
+                                                 red[v].ld, self.n_stats, C.stream_ptr()))
+        if not spec.member_fields:
+            return {}, groups
+        return {v: red[v] for v in self.output_vars}, groups
+
     def _download(self, out, agg):
         torch = self._torch
         compute = torch.cuda.current_stream()
-        staged = {v: out[v].to_device_cell_major() for v in self.output_vars}      # transposes run on the compute stream
+        if self.spec is None:
+            fields, groups = {v: out[v] for v in self.output_vars}, {}
+        else:
+            fields, groups = self._reduce(out)
+        staged = {v: f.to_device_cell_major() for v, f in fields.items()}      # transposes run on the compute stream
         ev = torch.cuda.Event()
         ev.record(compute)
         self.d2h.wait_event(ev)
@@ -248,7 +380,7 @@ class EnsembleRunner:
         with torch.cuda.stream(self.d2h):
             for v, dev in staged.items():
                 dev.record_stream(self.d2h)
-                h = C.host_pool.acquire((self.s.ncell, self.s.nmonths))
+                h = C.host_pool.acquire((self.s.ncell, self.ntime))
                 h.copy_(dev, non_blocking=True)
                 host[v] = h
                 self.d2h_bytes += h.numel() * 8
@@ -258,15 +390,53 @@ class EnsembleRunner:
                 h.copy_(agg, non_blocking=True)
                 host['basin_aggregates'] = h
                 self.d2h_bytes += h.numel() * 8
+            if groups:
+                host['group_sums'] = {}
+                for g, t in groups.items():
+                    t.record_stream(self.d2h)
+                    h = torch.empty(tuple(t.shape), dtype=torch.float64, pin_memory=True)
+                    h.copy_(t, non_blocking=True)
+                    host['group_sums'][g] = h
+                    self.d2h_bytes += h.numel() * 8
             done = torch.cuda.Event(enable_timing=self.timeline is not None)
             done.record(self.d2h)
         return host, done
+
+    # ---- across-member statistics -----------------------------------------------------------------------------------
+    def stats_partial(self):
+        """This runner's accumulators as a flat list [(sum, m2) of var 0, (min, max) of var 0, ...] (None before any
+        member): what `merge_stats` combines and `finalize_stats` turns into the statistics."""
+        if self._stats_state is None or self.n_stats == 0:
+            return None
+        return [t for v in self.output_vars for t in self._stats_state[v]]
+
+    def merge_stats(self, a, na, b, nb):
+        """Partial `a` of na members absorbs partial `b` of nb members (xan_ens_stats_merge, in place); returns a."""
+        for v in range(len(self.output_vars)):
+            C.check(C.lib().xan_ens_stats_merge(C.ptr(a[2 * v]), C.ptr(a[2 * v + 1]), C.ptr(b[2 * v]),
+                                                C.ptr(b[2 * v + 1]), self.s.ncell, self.ntime, self.s.ld, int(na),
+                                                int(nb), C.stream_ptr()))
+        return a
+
+    def finalize_stats(self, partial, n):
+        """{var: {stat: host ndarray [ncell, ntime]}} of the requested statistics over n members."""
+        torch, s, out = self._torch, self.s, {}
+        for k, v in enumerate(self.output_vars):
+            dev = {st: torch.empty((s.ncell, self.ntime), dtype=torch.float64, device='cuda') for st in self.spec.stats}
+            C.check(C.lib().xan_ens_stats_finalize(C.ptr(partial[2 * k]), C.ptr(partial[2 * k + 1]), s.ncell,
+                                                   self.ntime, s.ld, int(n), self.spec.ddof,
+                                                   *[C.ptr(dev.get(st)) for st in STATS], C.stream_ptr()))
+            out[v] = {st: t.cpu().numpy() for st, t in dev.items()}
+            self.d2h_bytes += sum(t.numel() * 8 for t in dev.values())
+        return out
 
     # ---- driver ----------------------------------------------------------------------------------------------------------
     def run(self, members):
         """Generator: yields (index, {variable: host ndarray [ncell, nmonths], 'basin_aggregates': [2, nmonths, n_basins]})
         in member order; the next members are being uploaded and a group of `group` members computed while the outputs of
-        the group before are handed out."""
+        the group before are handed out.  With a spec the grids are [ncell, ntime] (none without member_fields), the
+        result has 'group_sums': {scale: [ngroups, ntime]}, and each member is added to the across-member statistics
+        (`stats_partial` / `finalize_stats` once the generator is exhausted)."""
         torch = self._torch
         members = list(members)
         if not members:
@@ -275,7 +445,12 @@ class EnsembleRunner:
         n, depth, g = len(members), self.prefetch_depth, self.group
         # pinned output buffers in flight: the group being computed, the group before it on its way to the host, and the
         # results the caller still holds from the last hand-out - allocated before the pipeline starts, not inside it
-        C.host_pool.reserve((self.s.ncell, self.s.nmonths), min(3 * g, n + g) * len(self.output_vars))
+        if self.spec is None or self.spec.member_fields:
+            C.host_pool.reserve((self.s.ncell, self.ntime), min(3 * g, n + g) * len(self.output_vars))
+        self.n_stats = 0
+        if self.spec is not None and self.spec.stats and self._stats_state is None:
+            self._stats_state = {v: tuple(torch.empty((self.ntime, self.s.ld, 2), dtype=torch.float64, device='cuda')
+                                          for _ in range(2)) for v in self.output_vars}
         uploaded, next_up = {}, 0
         pending = []              # (index, host tensors, done event) of the members whose outputs are in flight
         computed = {}             # member -> completion event of its group's compute stage, to bound the uploads' run-ahead
@@ -328,36 +503,64 @@ class EnsembleRunner:
         done.synchronize()
         res = {}
         for v, h in host.items():
-            res[v] = C.host_pool.as_array(h) if v != 'basin_aggregates' else h.numpy()
+            if v == 'group_sums':
+                res[v] = {g: t.numpy() for g, t in h.items()}
+            else:
+                res[v] = C.host_pool.as_array(h) if v != 'basin_aggregates' else h.numpy()
         return k, res
 
 
-def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=True, on_result=None):
+def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=True, on_result=None, spec=None):
     """
     Run every member (this rank's share when torch.distributed is initialised: a contiguous block per rank,
     sharding.partition_members).
     Returns {member index: result dict}; with `on_result(index, result)` given the results are handed to it instead of
     being kept (a 64-member ensemble of 1,032 months is 2 x 36 GB of output).  On every rank the returned dict also has
     the key 'basin_aggregates': [n_members, 2, nmonths, n_basins] of ALL members (all-gather over NCCL).
+
+    `spec` (OutputSpec) reduces the outputs on the device before they are copied back; without it every member's
+    monthly grids come back as they are.  With it:
+      * a member's result holds the grids {var: [ncell, ntime]} (ntime = nyears with yearly output) only if
+        spec.member_fields, and 'group_sums': {scale: [ngroups, ntime]};
+      * the returned dict has 'group_sums': {scale: [n_members, ngroups, ntime]} of all members on every rank, and on
+        rank 0 'ensemble_stats': {var: {stat: [ncell, ntime]}, 'n_members': N}.
+    The statistics are accumulated on the device member by member (fp64 accumulators of 32 B per cell and time step
+    and variable: 2.2 GB per monthly variable at 67,420 cells x 1,032 months); each rank keeps the partial of its
+    members and rank 0 merges them in rank order (Chan et al.).  The result is deterministic for a given number of
+    ranks; min / max do not depend on it, mean and std may differ in the last bits between rank counts.
     """
     torch = C.torch_cuda()
     import torch.distributed as dist
     members = list(members)
     dist_on = dist.is_available() and dist.is_initialized()
     rank, world = (dist.get_rank(), dist.get_world_size()) if dist_on else (0, 1)
-    mine = [int(i) for i in sharding.partition_members(len(members), world)[rank]]
-    runner = EnsembleRunner(statics, output_vars, aggregates)
+    parts = sharding.partition_members(len(members), world)
+    mine = [int(i) for i in parts[rank]]
+    runner = EnsembleRunner(statics, output_vars, aggregates, spec=spec)
     results = {}
     agg_local = torch.zeros((len(mine), 2, statics.nmonths, statics.n_basins), dtype=torch.float64)
+    groups = spec.group_sums if spec is not None else ()
+    grp_local = {g: torch.zeros((len(mine), statics.group_table(g)[2], runner.ntime), dtype=torch.float64)
+                 for g in groups}
     for j, res in runner.run([members[i] for i in mine]):
         if aggregates:
             agg_local[j] = torch.from_numpy(res['basin_aggregates'])
+        for g in groups:
+            grp_local[g][j] = torch.from_numpy(res['group_sums'][g])
         if on_result is not None:
             on_result(mine[j], res)
         else:
             results[mine[j]] = res
-    if aggregates:      # the only collective: every rank gets the basin aggregates of all members
+    if aggregates:      # every rank gets the basin aggregates of all members
         results['basin_aggregates'] = sharding.gather_ragged_rows(mine, agg_local.cuda(), len(members)).cpu().numpy()
+    if groups:
+        results['group_sums'] = {g: sharding.gather_ragged_rows(mine, grp_local[g].cuda(), len(members)).cpu().numpy()
+                                 for g in groups}
+    if spec is not None and spec.stats and members:
+        partial = sharding.fold_to_rank0(runner.stats_partial(), [len(p) for p in parts], runner.merge_stats)
+        if rank == 0:
+            results['ensemble_stats'] = runner.finalize_stats(partial, len(members))
+            results['ensemble_stats']['n_members'] = len(members)
     results['stats'] = {'h2d_bytes': runner.h2d_bytes, 'd2h_bytes': runner.d2h_bytes, 'members_local': len(mine)}
     if runner.timeline:      # ms relative to the first upload: (h2d start, end), (compute start, end), outputs on the host
         torch.cuda.synchronize()

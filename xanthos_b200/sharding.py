@@ -11,8 +11,9 @@ The hot path shards without any exchange inside the time loop (SURVEY.md section
                                       (`basins_closed_under_flow`); Penman-Monteith needs the air
                                       temperature of the previous cell id, a one-column halo of an INPUT.
 
-The only collective is a gather of small results at the end of a step (`gather_stack`), NCCL on GPUs,
-gloo in the CPU tests.
+The only exchanges are a gather of small results at the end of a step (`gather_stack`, `gather_ragged_rows`) and the
+rank-order fold of partial results onto rank 0 (`fold_to_rank0`, the ensemble statistics), NCCL on GPUs, gloo in the
+CPU tests.
 """
 
 import numpy as np
@@ -129,6 +130,37 @@ def gather_stack(local, group=None):
     parts = [torch.empty_like(local) for _ in range(dist.get_world_size(group))]
     dist.all_gather(parts, local.contiguous(), group=group)
     return torch.stack(parts, dim=0)
+
+
+def fold_to_rank0(partial, counts, merge):
+    """
+    Rank-order fold of per-rank partial results onto rank 0 (point-to-point: NCCL for cuda tensors, gloo for cpu).
+    partial: this rank's list of tensors (None on a rank with counts[rank] == 0); counts: items per rank;
+    merge(a, na, b, nb) combines partial a of na items with partial b of nb items and returns the result.
+    Rank 0 returns merge(...merge(merge(p0, c0, p1, c1), c0 + c1, p2, c2)...), skipping ranks without items (None if
+    no rank has any); the other ranks send their partial and return None.  Single-process runs return `partial`.
+    The order is fixed, so the result is deterministic for a given world size.
+    """
+    import torch
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
+        return partial
+    rank = dist.get_rank()
+    if rank != 0:
+        if counts[rank] > 0:
+            for t in partial:
+                dist.send(t.contiguous(), dst=0)
+        return None
+    acc, n = partial, counts[0]
+    for r in range(1, len(counts)):
+        if counts[r] == 0:
+            continue
+        recv = [torch.empty_like(t) for t in acc]
+        for t in recv:
+            dist.recv(t, src=r)
+        acc = merge(acc, n, recv, counts[r])
+        n += counts[r]
+    return acc
 
 
 def gather_ragged_rows(local_rows, local_values, n_rows, group=None):

@@ -77,6 +77,23 @@ def test_abcd_spinup_too_short_raises():
                            np.nan_to_num(case['tmin']), case['abcd_pars'], case['nmonths'], 24)
 
 
+def test_kge_distance_of_a_constant_series_is_nan():
+    """The KGE correlation of the reference is np.corrcoef, which is NaN when either series is constant (zero
+    variance) and keeps that NaN through its np.clip: the distance is NaN, not a finite value from r = -1."""
+    from oracle.calibrate import kge_distance
+    rng = np.random.default_rng(0)
+    varying = rng.uniform(0.5, 2.0, 48)
+    cases = [(np.zeros(48), varying),          # modelled == 0: every cell of the basin has missing forcing
+             (varying, np.ones(48)),           # observed == 1
+             (varying, np.zeros(48))]          # observed == 0: a dry gauge
+    with np.errstate(invalid='ignore', divide='ignore'):
+        for mod, obs in cases:
+            assert np.isnan(np.corrcoef(obs, mod)[1, 0])
+            assert np.isnan(kge_distance(mod, obs))
+        # a correlation of 1 is kept (clipped if it rounds above 1): relvar = bias = 2 exactly
+        assert kge_distance(varying, 0.5 * varying) == pytest.approx(np.sqrt(2.0), rel=1e-12)
+
+
 @pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
 def test_oracle_matches_live_reference():
     case = build_case(nrow=20, ncol=40, ncell=180, n_basins=5, seed=77, start_yr=2003, end_yr=2005,

@@ -457,7 +457,8 @@ __global__ void __launch_bounds__(KGE_NT)
         const double relvar = sd_m / sd_o;
         const double bias = mean_m / mean_o;
         double r = cov / sqrt(vm * vo);
-        r = fmin(fmax(r, -1.0), 1.0);   // np.corrcoef clips to [-1, 1]
+        // np.corrcoef clips to [-1, 1] with np.clip, which keeps NaN (a constant series): fmax(NaN, -1) would give -1
+        r = r < -1.0 ? -1.0 : (r > 1.0 ? 1.0 : r);
         ed_out[(size_t)slot * npar + p] =
             sqrt(((r - 1) * (r - 1)) + ((relvar - 1) * (relvar - 1)) + ((bias - 1) * (bias - 1)));
     }
@@ -640,7 +641,7 @@ __global__ void __launch_bounds__(64)
         const double relvar = sd_m / sd_o;
         const double bias = mean_m / mean_o;
         double r = cov / sqrt(vm * vo);
-        r = fmin(fmax(r, -1.0), 1.0);   // np.corrcoef clips to [-1, 1]
+        r = r < -1.0 ? -1.0 : (r > 1.0 ? 1.0 : r);   // np.clip keeps NaN, as in abcd_kge_kernel
         ed_out[(size_t)slot * npar + p] =
             sqrt(((r - 1) * (r - 1)) + ((relvar - 1) * (relvar - 1)) + ((bias - 1) * (bias - 1)));
     }

@@ -283,6 +283,15 @@ int xan_ens_quantiles(const double *d_x, long long member_stride, int n, int nce
 int xan_drought_stats(const double *d_hydro, const double *d_thresh, int ncell, int nmonths, int ld,
                       int nthresh, int ld_thresh, double *d_severity, double *d_intensity,
                       double *d_duration, void *stream);
+/* The same scan with optional outputs (the ensemble runner's drought statistics).  Severity / intensity /
+ * duration as xan_drought_stats when all three are given, skipped when all three are null.  With d_count and
+ * d_summary (both or neither): d_count[t][c] += (hydro < threshold) for every month (int32 [nmonths][ld], the
+ * members in drought so far), and d_summary[4][ld] = the member's drought months (D > 0).sum(0), events
+ * (D == 1).sum(0), longest duration D.max(0) and peak severity S.max(0) (NaN if any severity is NaN, like
+ * np.max).  At least one of the two groups is required. */
+int xan_drought_scan(const double *d_hydro, const double *d_thresh, int ncell, int nmonths, int ld, int nthresh,
+                     int ld_thresh, double *d_severity, double *d_intensity, double *d_duration, int *d_count,
+                     double *d_summary, void *stream);
 /* DroughtStats.getthresh (drought_stats.py:150-171): numpy.percentile(..., method "linear") over the
  * ntime / nper samples of every (period, cell); the caller passes numpy's virtual index
  * ((n - 1) q, split into floor and fraction).  d_out [nper][ld_out]. */

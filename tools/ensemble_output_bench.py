@@ -6,13 +6,16 @@ End-to-end cost of the ensemble runner's output options on the bench world (67,4
   B  yearly + km3 + basin / country / region sums + mean / std / min / max, member grids copied back (yearly)
   C  as B without member grids (group sums per member, statistics once at the end)
   Q  as C plus the across-member quantiles (0.05, 0.5, 0.95) of every variable
+  D  as C plus drought statistics of q with per-member thresholds over the first 30 years (DroughtSpec)
 
-at config-1 length (1971-2000, 360 months) with 20 members per rank, and leg C at config 5 (64 members, 2015-2100,
-1,032 months).  Forcing values are single precision and cross the link as float32, as in bench.py's end-to-end leg.
+at config-1 length (1971-2000, 360 months) with 20 members per rank, and legs C and D at config 5 (64 members,
+2015-2100, 1,032 months).  Forcing values are single precision and cross the link as float32, as in bench.py's end-to-end leg.
 Each leg: one warm-up run, then the median of five runs (wall time of run_ensemble, max over ranks; every run listed).
 Also measured: the across-member statistics update kernel (xan_ens_stats_update) at config-5 size with CUDA events,
 and, on rank 0, that the merged statistics of leg C equal those of all members run by one process.  With leg Q: the
 quantile kernel (xan_ens_quantiles) alone over 64 members of yearly (86) and monthly (1,032) fields, CUDA events.
+With leg D: the drought scan (xan_drought_scan) alone at config-5 size, accumulation only and with severity /
+intensity / duration, CUDA events.
 `--legs` picks the legs.
 
     python tools/ensemble_output_bench.py --out profiles/ensemble_output_n1.json
@@ -180,12 +183,56 @@ def quantile_kernel(ncell, ntime, n=64, launches=20):
             'gb_per_s': round((read + written) / (ms * 1e-3) / 1e9, 1)}
 
 
+DROUGHT_YEARS = 30                # per-member thresholds from the first 30 years of the run, as a 1971-2000 baseline
+
+
+def drought_spec(sy):
+    from xanthos_b200 import ensemble as ens
+    return ens.DroughtSpec('q', threshold_years=(sy, sy + DROUGHT_YEARS - 1))
+
+
+def drought_kernel(ncell, nmonths, launches=20):
+    """xan_drought_scan over a [nmonths][ld] field with 12 threshold rows, CUDA events around `launches` back-to-back
+    launches after two warm-up launches, accumulation only and accumulation plus severity / intensity / duration.  The
+    field and the counts (12 B per cell-month) are far larger than the L2.  Algorithmic bytes per cell-month: the
+    field read (8), the count read and written (4 + 4) and with the fields 24 B written; per cell the 12 threshold
+    rows read once (96) and the summary written (32)."""
+    import torch
+    from xanthos_b200 import _cuda as C
+    from xanthos_b200.drought.drought_stats import drought_scan_device
+    ld = C.padded_ld(ncell)
+    g = torch.Generator(device='cuda').manual_seed(5)
+    hydro = torch.rand((nmonths, ld), dtype=torch.float64, device='cuda', generator=g)
+    th = torch.full((12, ncell), 0.1, dtype=torch.float64, device='cuda')       # about 10 % of the months are dry
+    count = torch.zeros((nmonths, ld), dtype=torch.int32, device='cuda')
+    summary = torch.empty((4, ld), dtype=torch.float64, device='cuda')
+    sid = [torch.empty((nmonths, ld), dtype=torch.float64, device='cuda') for _ in range(3)]
+    out = {'ncell': ncell, 'nmonths': nmonths, 'launches': launches, 'dry_fraction': 0.1}
+    for name, fields in (('accumulate', None), ('accumulate_and_fields', sid)):
+        for _ in range(2):
+            drought_scan_device(hydro, ncell, th, fields, count, summary)
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(launches):
+            drought_scan_device(hydro, ncell, th, fields, count, summary)
+        e1.record()
+        e1.synchronize()
+        ms = e0.elapsed_time(e1) / launches
+        nbytes = (16 + (24 if fields else 0)) * ncell * nmonths + (96 + 32) * ncell
+        gbs = nbytes / (ms * 1e-3) / 1e9
+        out[name] = {'ms_per_launch': round(ms, 4), 'algorithmic_bytes': nbytes, 'gb_per_s': round(gbs, 1),
+                     'frac_of_6551_gbs_copy_peak': round(gbs / 6551.0, 3)}
+    del hydro, count, sid
+    torch.cuda.empty_cache()
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--members', type=int, default=20, help='members per rank at config-1 length')
     ap.add_argument('--reps', type=int, default=5)
     ap.add_argument('--config5-members', type=int, default=64, help='0 skips the config-5 leg')
-    ap.add_argument('--legs', default='A,B,C,Q', help='comma-separated subset of A, B, C, Q')
+    ap.add_argument('--legs', default='A,B,C,Q', help='comma-separated subset of A, B, C, Q, D')
     ap.add_argument('--rounds', type=int, default=1, help='the legs in turn this many times (drift shows between '
                                                           'rounds); the last round is reported per leg')
     ap.add_argument('--out', default=None)
@@ -202,7 +249,9 @@ def main():
     spec_b = dict(output_in_year=True, output_unit='km3', group_sums=ens.GROUP_SCALES, stats=ens.STATS)
     legs = {'A': dict(), 'B': dict(aggregates=False, spec=ens.OutputSpec(**spec_b)),
             'C': dict(aggregates=False, spec=ens.OutputSpec(member_fields=False, **spec_b)),
-            'Q': dict(aggregates=False, spec=ens.OutputSpec(member_fields=False, quantiles=QUANTILE_LEVELS, **spec_b))}
+            'Q': dict(aggregates=False, spec=ens.OutputSpec(member_fields=False, quantiles=QUANTILE_LEVELS, **spec_b)),
+            'D': dict(aggregates=False, spec=ens.OutputSpec(member_fields=False, drought=drought_spec(bench.START_YR),
+                                                            **spec_b))}
     legs_order = [k for k in args.legs.split(',') if k in legs]
     legs = {k: legs[k] for k in legs_order}
     out = {'card': card(), 'world_size': world_size, 'transport': 'float32 (single-precision forcing values)',
@@ -255,10 +304,16 @@ def main():
         if 'Q' in legs:
             out['quantile_kernel'] = {'yearly': quantile_kernel(bench.NCELL, 86),
                                       'monthly': quantile_kernel(bench.NCELL, 1032)}
-    if args.config5_members > 0 and 'C' in legs:
+        if 'D' in legs:
+            out['drought_kernel_config5'] = drought_kernel(bench.NCELL, 1032)
+    c5 = [k for k in ('C', 'D') if k in legs]
+    if args.config5_members > 0 and c5:
         st, mem_a, mem_b = setup(2015, 2100)
         members = [mem_a if k % 2 == 0 else mem_b for k in range(args.config5_members)]
-        out['config5']['C'], _ = time_leg(st, members, legs['C'], world_size, args.reps)
+        if 'D' in legs:
+            legs['D'] = dict(legs['D'], spec=ens.OutputSpec(member_fields=False, drought=drought_spec(2015), **spec_b))
+        for name in c5:
+            out['config5'][name], _ = time_leg(st, members, legs[name], world_size, args.reps)
     if rank == 0:
         line = json.dumps(out)
         print(line, flush=True)

@@ -21,6 +21,7 @@ XAN_OK, XAN_E_INVALID, XAN_E_CUDA, XAN_E_SPINUP, XAN_E_NOMEM = 0, -1, -2, -3, -4
 MRTM_AUTO, MRTM_GRID, MRTM_TREE, MRTM_SKEW = 0, 1, 2, 3
 PM_MAX_CLASSES = 32
 ENS_MAX_MEMBERS, ENS_MAX_LEVELS = 256, 64      # XAN_ENS_MAX_MEMBERS / XAN_ENS_MAX_LEVELS (xan_ens_quantiles)
+DROUGHT_MAX_YEARS = 1024                        # MAX_YEARS of xan_drought_thresholds: samples per (period, cell)
 
 
 class ValidationException(Exception):
@@ -77,6 +78,7 @@ SIGNATURES = {
     'xan_agg_to_year': (c_int, [_P, _P, c_int, c_int, c_int, c_int, _P]),
     'xan_basin_sum': (c_int, [_P, _P, _P, c_int, c_int, _P, _P]),
     'xan_drought_stats': (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P]),
+    'xan_drought_scan': (c_int, [_P, _P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     'xan_drought_thresholds': (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_double, _P, c_int, _P]),
     'xan_group_sum': (c_int, [_P, _P, _P, c_int, c_int, c_int, _P, _P]),
     'xan_year_sum_scaled': (c_int, [_P, _P, c_int, c_int, c_int, _P, _P]),
@@ -99,7 +101,7 @@ KERNELS_PER_CALL = {
     'xan_to_month_major': 1, 'xan_to_month_major_f32': 1, 'xan_to_cell_major': 1, 'xan_hs_pet': 2, 'xan_thornthwaite_pet': 2,
     'xan_thornthwaite_daylight': 1, 'xan_pm_pet': 1, 'xan_abcd_run': 3, 'xan_abcd_kge_batch': 1,
     'xan_mrtm_route': 1, 'xan_mrtm_route_batch': 1, 'xan_hargreaves_pet': 1, 'xan_gwam_run': 1, 'xan_agg_to_year': 1, 'xan_basin_sum': 1,
-    'xan_drought_stats': 1, 'xan_drought_thresholds': 1, 'xan_group_sum': 1, 'xan_year_sum_scaled': 1,
+    'xan_drought_stats': 1, 'xan_drought_scan': 1, 'xan_drought_thresholds': 1, 'xan_group_sum': 1, 'xan_year_sum_scaled': 1,
     'xan_scale_cells': 1, 'xan_ens_stats_update': 1, 'xan_ens_stats_merge': 1, 'xan_ens_stats_finalize': 1,
     'xan_ens_quantiles': 1, 'xan_de_init': 1, 'xan_de_trial': 1, 'xan_de_select': 1,
 }

@@ -1,6 +1,7 @@
 // Post-processing scans on the device-resident [month][cell] fields (SURVEY.md section 8, row f3).
 //
-//   * drought_stats_kernel      - DroughtStats.droughtstats   (xanthos/drought/drought_stats.py:85-148)
+//   * drought_scan_kernel       - DroughtStats.droughtstats   (xanthos/drought/drought_stats.py:85-148), and the
+//                                 ensemble runner's drought counts and member summaries in the same scan
 //   * drought_thresholds_kernel - DroughtStats.getthresh      (drought_stats.py:150-171, numpy.percentile "linear")
 //   * group_sum_kernel          - Aggregation_Map             (xanthos/diagnostics/time_series.py:126-138) and the
 //                                 basin aggregation of AccessibleWater (xanthos/accessible/accessible.py:41-51)
@@ -19,26 +20,38 @@ namespace xan {
 // K <= 12 threshold rows stay in L2 / L1) + 24 B written per cell-month.
 // Quirk kept: month 0 uses threshold row 0 and intensity == severity there (drought_stats.py:121-123);
 // later months use row t % K (:130).
+//
+// FIELDS writes S / I / D.  ACCUM is the ensemble accumulation: count[t][c] += dry (int32, the number of members in
+// drought so far) and, per cell, the member summary [4][ld] = (D > 0).sum(0), (D == 1).sum(0), D.max(0), S.max(0)
+// (NaN-propagating like np.max).  Without FIELDS the traffic is 8 B read + at most 4 + 4 B of count per cell-month:
+// the count is added in L2 by a reduction without return value, only in dry months.  The accumulation arguments
+// come last, so FIELDS-only compiles to the code of the kernel before it had them (same SASS, 60 registers).
 // ---------------------------------------------------------------------------------------------
 constexpr int DS_BATCH = 8;   // months loaded ahead of the scan (the scan itself is a dependent chain per cell)
 
+template <bool FIELDS, bool ACCUM>
 __global__ void __launch_bounds__(128)
-    drought_stats_kernel(const double *__restrict__ hydro, const double *__restrict__ thresh, int ncell, int nmonths,
-                         int ld, int ld_t, int nthresh, double *__restrict__ S, double *__restrict__ I,
-                         double *__restrict__ D) {
+    drought_scan_kernel(const double *__restrict__ hydro, const double *__restrict__ thresh, int ncell, int nmonths,
+                        int ld, int ld_t, int nthresh, double *__restrict__ S, double *__restrict__ I,
+                        double *__restrict__ D, int *__restrict__ count, double *__restrict__ summary) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= ncell) return;
     double s = 0.0, d = 0.0;
-    for (int t0 = 0; t0 < nmonths; t0 += DS_BATCH) {
-        double h[DS_BATCH], th[DS_BATCH];
+    int n_dry = 0, n_events = 0;
+    float longest = 0.0f;           // a whole number of months: exact in float, one register fewer
+    double peak = -INFINITY;        // np.max: the first severity replaces it (a -inf severity leaves it equal)
+    // both groups: one month fewer in flight keeps the kernel within 64 registers (8 blocks per SM, as FIELDS alone)
+    constexpr int B = FIELDS && ACCUM ? DS_BATCH - 1 : DS_BATCH;
+    for (int t0 = 0; t0 < nmonths; t0 += B) {
+        double h[B], th[B];
 #pragma unroll
-        for (int k = 0; k < DS_BATCH; ++k) {                      // all loads of the batch in flight together
+        for (int k = 0; k < B; ++k) {                      // all loads of the batch in flight together
             const int t = min(t0 + k, nmonths - 1);
             h[k] = ldg_stream(hydro + (size_t)t * ld + c);
             th[k] = thresh[(size_t)(t % nthresh) * ld_t + c];
         }
 #pragma unroll
-        for (int k = 0; k < DS_BATCH; ++k) {
+        for (int k = 0; k < B; ++k) {
             const int t = t0 + k;
             if (t >= nmonths) break;
             const bool dry = h[k] < th[k];                          // false for NaN, like numpy
@@ -53,10 +66,25 @@ __global__ void __launch_bounds__(128)
                 s = dry ? s + deficit : 0.0;
                 it = dry ? s / d : 0.0;
             }
-            stg_stream(S + (size_t)t * ld + c, s);
-            stg_stream(I + (size_t)t * ld + c, it);
-            stg_stream(D + (size_t)t * ld + c, d);
+            if constexpr (FIELDS) {
+                stg_stream(S + (size_t)t * ld + c, s);
+                stg_stream(I + (size_t)t * ld + c, it);
+                stg_stream(D + (size_t)t * ld + c, d);
+            }
+            if constexpr (ACCUM) {
+                if (dry) atomicAdd(count + (size_t)t * ld + c, 1);   // result unused: a RED, no register, no wait
+                n_dry += dry ? 1 : 0;
+                n_events += (d == 1.0) ? 1 : 0;
+                longest = fmaxf(longest, (float)d);                 // d is never NaN
+                if (!isnan(peak) && !(s <= peak)) peak = s;         // a NaN severity sticks, as in np.max
+            }
         }
+    }
+    if constexpr (ACCUM) {
+        summary[c] = (double)n_dry;
+        summary[(size_t)ld + c] = (double)n_events;
+        summary[2 * (size_t)ld + c] = (double)longest;
+        summary[3 * (size_t)ld + c] = peak;
     }
 }
 
@@ -172,8 +200,37 @@ int xan_drought_stats(const double *d_hydro, const double *d_thresh, int ncell, 
     XAN_REQUIRE(ncell > 0 && nmonths > 0 && nthresh > 0 && ld >= ncell && ld_thresh >= ncell,
                 "xan_drought_stats: bad shape ncell=%d nmonths=%d nthresh=%d ld=%d ld_thresh=%d", ncell, nmonths,
                 nthresh, ld, ld_thresh);
-    drought_stats_kernel<<<ceil_div(ncell, 128), 128, 0, (cudaStream_t)stream>>>(
-        d_hydro, d_thresh, ncell, nmonths, ld, ld_thresh, nthresh, d_severity, d_intensity, d_duration);
+    drought_scan_kernel<true, false><<<ceil_div(ncell, 128), 128, 0, (cudaStream_t)stream>>>(
+        d_hydro, d_thresh, ncell, nmonths, ld, ld_thresh, nthresh, d_severity, d_intensity, d_duration, nullptr,
+        nullptr);
+    XAN_CUDA_CHECK(cudaGetLastError());
+    return XAN_OK;
+}
+
+int xan_drought_scan(const double *d_hydro, const double *d_thresh, int ncell, int nmonths, int ld, int nthresh,
+                     int ld_thresh, double *d_severity, double *d_intensity, double *d_duration, int *d_count,
+                     double *d_summary, void *stream) {
+    const bool fields = d_severity || d_intensity || d_duration, accum = d_count || d_summary;
+    XAN_REQUIRE(d_hydro && d_thresh, "xan_drought_scan: null pointer");
+    XAN_REQUIRE(!fields || (d_severity && d_intensity && d_duration),
+                "xan_drought_scan: severity, intensity and duration are written together");
+    XAN_REQUIRE(!accum || (d_count && d_summary), "xan_drought_scan: count and summary are accumulated together");
+    XAN_REQUIRE(fields || accum, "xan_drought_scan: no output requested");
+    XAN_REQUIRE(ncell > 0 && nmonths > 0 && nthresh > 0 && ld >= ncell && ld_thresh >= ncell,
+                "xan_drought_scan: bad shape ncell=%d nmonths=%d nthresh=%d ld=%d ld_thresh=%d", ncell, nmonths,
+                nthresh, ld, ld_thresh);
+    const dim3 grid(ceil_div(ncell, 128));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (fields && accum)
+        drought_scan_kernel<true, true><<<grid, 128, 0, st>>>(d_hydro, d_thresh, ncell, nmonths, ld, ld_thresh, nthresh,
+                                                              d_severity, d_intensity, d_duration, d_count, d_summary);
+    else if (fields)
+        drought_scan_kernel<true, false><<<grid, 128, 0, st>>>(d_hydro, d_thresh, ncell, nmonths, ld, ld_thresh,
+                                                               nthresh, d_severity, d_intensity, d_duration, nullptr,
+                                                               nullptr);
+    else
+        drought_scan_kernel<false, true><<<grid, 128, 0, st>>>(d_hydro, d_thresh, ncell, nmonths, ld, ld_thresh,
+                                                               nthresh, nullptr, nullptr, nullptr, d_count, d_summary);
     XAN_CUDA_CHECK(cudaGetLastError());
     return XAN_OK;
 }

@@ -65,6 +65,20 @@ def droughtstats_device(hydro, ngrid, thresh):
     return S, I, D
 
 
+def drought_scan_device(hydro, ngrid, thresh, sid=None, count=None, summary=None):
+    """xan_drought_scan: hydro cuda [ntime, ld], thresh cuda [K, ld_t]; sid = (S, I, D) cuda [ntime, ld] written as
+    droughtstats_device writes them; count int32 cuda [ntime, ld] += months in drought and summary cuda [4, ld] = the
+    drought months, events, longest duration and peak severity of every cell.  At least one of sid / count."""
+    ntime, ld = int(hydro.shape[0]), int(hydro.shape[1])
+    if int(thresh.shape[1]) < ngrid or thresh.stride(1) != 1:
+        raise C.ValidationException("drought thresholds {} (strides {}) are not rows of at least {} cells".format(
+            tuple(thresh.shape), thresh.stride(), ngrid))
+    S, I, D = sid if sid is not None else (None, None, None)
+    C.check(C.lib().xan_drought_scan(C.ptr(hydro), C.ptr(thresh), ngrid, ntime, ld, int(thresh.shape[0]),
+                                     int(thresh.stride(0)), C.ptr(S), C.ptr(I), C.ptr(D), C.ptr(count), C.ptr(summary),
+                                     C.stream_ptr()))
+
+
 class DroughtStats:
     """Analyze drought impacts based on runoff or soil moisture (Sheffield and Wood 2008)."""
 

@@ -41,6 +41,78 @@ FORCING = PM_FORCING + ('precip', 'tmin')
 OUTPUTS = ('pet', 'aet', 'q', 'soilmoisture', 'chstorage', 'avgchflow')
 GROUP_SCALES = ('basin', 'country', 'region')
 STATS = ('mean', 'std', 'min', 'max')
+DROUGHT_VARS = ('q', 'soilmoisture')
+DROUGHT_SUMMARY = ('drought_months', 'events', 'longest_duration', 'peak_severity')
+DROUGHT_FIELDS = ('severity', 'intensity', 'duration')
+
+
+class DroughtSpec:
+    """
+    Drought statistics of every member, the [Drought] section of a configuration (ConfigReader.configure_drought_stats)
+    applied to the member's monthly mm field of `var` ('q' or 'soilmoisture'), whatever the spec's yearly / km3 options:
+
+      thresholds       host array [K, ncell]: the thresholds of every member (drought_thresholds of the .ini), row t % K
+                       for month t; staged on the device once
+      threshold_years  (start, end) when no thresholds are given: each member's thresholds are its 10th percentile per
+                       period over the months DroughtStats.calculate_thresholds takes (the slice end
+                       (end + 1 - start) * 12 is an index, as in the reference), with `nper` periods
+      fields           also return the member's severity / intensity / duration grids [ncell, nmonths]
+
+    Every member gets its summary per cell - drought months, events, longest duration, peak severity - and the runner
+    counts per cell and month how many members are in drought (a month is dry when the field is below the threshold;
+    NaN is never dry).  The severity / intensity / duration and the thresholds are bitwise DroughtStats' on the member.
+    """
+
+    def __init__(self, var='q', thresholds=None, threshold_years=None, nper=12, fields=False):
+        var = str(var).lower()
+        if var not in DROUGHT_VARS:
+            raise C.ValidationException("drought variable must be one of {}, not {!r}".format(DROUGHT_VARS, var))
+        if (thresholds is None) == (threshold_years is None):
+            raise C.ValidationException("give drought thresholds or threshold_years (one of the two)")
+        if int(nper) != nper or nper < 1:
+            raise C.ValidationException("nper must be a positive integer, not {!r}".format(nper))
+        self.var, self.nper, self.fields = var, int(nper), bool(fields)
+        self.thresholds = self.threshold_years = None
+        if thresholds is not None:
+            th = np.array(thresholds, dtype=np.float64, order='C')      # staged as [K][ncell] rows
+            if th.ndim != 2 or th.shape[0] < 1:
+                raise C.ValidationException("drought thresholds must be [K, ncell] with K >= 1, not {}".format(th.shape))
+            self.thresholds = th
+        else:
+            years = tuple(int(y) for y in threshold_years)
+            if len(years) != 2:
+                raise C.ValidationException("threshold_years must be (start, end), not {!r}".format(threshold_years))
+            self.threshold_years = years
+
+    def reference_months(self, start_year, end_year):
+        """(first, end) of the months the per-member thresholds are computed from, in a run of start_year .. end_year
+        (DroughtStats.calculate_thresholds' slice); raises ValidationException where the reference would fail."""
+        sy, ey = self.threshold_years
+        if sy < start_year or ey > end_year:
+            raise C.ValidationException("drought threshold years {} - {} are outside the run {} - {}".format(
+                sy, ey, start_year, end_year))
+        nmonths = (end_year - start_year + 1) * 12
+        first, end = (sy - start_year) * 12, (ey + 1 - sy) * 12
+        n = len(range(nmonths)[first:end])
+        if n == 0 or n % self.nper or n // self.nper > C.DROUGHT_MAX_YEARS:
+            raise C.ValidationException(
+                "drought reference period: months [{}:{}] of the run give {} months, not a positive multiple of {} "
+                "periods of at most {} years".format(first, end, n, self.nper, C.DROUGHT_MAX_YEARS))
+        return first, end
+
+    def validate(self, ncell, start_year, end_year):
+        """Refuses a spec that cannot run on ncell cells and the years start_year .. end_year."""
+        if self.thresholds is not None:
+            if self.thresholds.shape[1] != ncell:
+                raise C.ValidationException("drought thresholds have {} cells, the run {}".format(
+                    self.thresholds.shape[1], ncell))
+        else:
+            self.reference_months(start_year, end_year)
+
+    def __repr__(self):
+        src = ('thresholds=<{} x {}>'.format(*self.thresholds.shape) if self.thresholds is not None
+               else 'threshold_years={}'.format(self.threshold_years))
+        return 'DroughtSpec(var={!r}, {}, nper={}, fields={})'.format(self.var, src, self.nper, self.fields)
 
 
 class OutputSpec:
@@ -58,13 +130,14 @@ class OutputSpec:
                       variable; std with `ddof` like numpy.std
       quantiles       levels in [0, 1], in the order given: numpy.quantile(members, levels, axis=0) (method 'linear')
                       per (cell, time step) of every output variable; the median is quantiles=(0.5,)
+      drought         DroughtSpec: drought statistics of every member and the across-member drought frequency
 
     Every member's grids and group sums are bit-identical to what OutWriter.write / write_aggregates produce from that
     member's monthly outputs.  chstorage is never written through OutWriter: it is rejected with yearly or km3 output.
     """
 
     def __init__(self, output_in_year=False, output_unit='mm', group_sums=(), member_fields=True, stats=(), ddof=0,
-                 quantiles=()):
+                 quantiles=(), drought=None):
         if output_unit not in ('mm', 'km3'):
             raise C.ValidationException("output_unit must be 'mm' or 'km3', not {!r}".format(output_unit))
         group_sums, stats = tuple(group_sums), tuple(stats)
@@ -79,26 +152,47 @@ class OutputSpec:
                 or len(quantiles) > C.ENS_MAX_LEVELS):
             raise C.ValidationException("quantile levels must be distinct, in [0, 1] and at most {}, not {}".format(
                 C.ENS_MAX_LEVELS, quantiles))
-        self.quantiles = quantiles
+        if drought is not None and not isinstance(drought, DroughtSpec):
+            raise C.ValidationException("drought must be a DroughtSpec, not {!r}".format(drought))
+        self.quantiles, self.drought = quantiles, drought
         self.output_in_year, self.output_unit = bool(output_in_year), output_unit
         self.group_sums, self.member_fields, self.stats, self.ddof = group_sums, bool(member_fields), stats, int(ddof)
 
     @classmethod
-    def from_settings(cls, settings, member_fields=True, stats=(), ddof=0, quantiles=()):
+    def from_settings(cls, settings, member_fields=True, stats=(), ddof=0, quantiles=(), drought=False):
         """The output options of a parsed configuration (data_reader.ini_reader.ConfigReader): OutputInYear,
-        OutputUnit and the AggregateRunoffBasin / Country / GCAMRegion flags."""
+        OutputUnit and the AggregateRunoffBasin / Country / GCAMRegion flags; with drought=True also its [Drought]
+        section (drought_var, and drought_thresholds loaded with np.load or the threshold years and nper)."""
         unit = int(settings.OutputUnit)
         if unit not in (0, 1):
             raise C.ValidationException("OutputUnit must be 0 (mm) or 1 (km3), not {}".format(unit))
+        dspec = None
+        if drought:
+            if getattr(settings, 'drought_var', None) is None:
+                raise C.ValidationException("drought output requested, but the configuration has no [Drought] section "
+                                            "(CalculateDroughtStats = 1)")
+            if settings.drought_thresholds is not None:
+                dspec = DroughtSpec(settings.drought_var, thresholds=np.load(settings.drought_thresholds))
+            else:
+                dspec = DroughtSpec(settings.drought_var, nper=settings.threshold_nper,
+                                    threshold_years=(settings.threshold_start_year, settings.threshold_end_year))
         flags = (settings.AggregateRunoffBasin, settings.AggregateRunoffCountry, settings.AggregateRunoffGCAMRegion)
         return cls(output_in_year=bool(int(settings.OutputInYear)), output_unit=('mm', 'km3')[unit],
                    group_sums=tuple(g for g, f in zip(GROUP_SCALES, flags) if int(f)), member_fields=member_fields,
-                   stats=stats, ddof=ddof, quantiles=quantiles)
+                   stats=stats, ddof=ddof, quantiles=quantiles, drought=dspec)
 
     def __repr__(self):
         return ('OutputSpec(output_in_year={}, output_unit={!r}, group_sums={}, member_fields={}, stats={}, ddof={}, '
-                'quantiles={})'.format(self.output_in_year, self.output_unit, self.group_sums, self.member_fields,
-                                       self.stats, self.ddof, self.quantiles))
+                'quantiles={}{})'.format(self.output_in_year, self.output_unit, self.group_sums, self.member_fields,
+                                         self.stats, self.ddof, self.quantiles,
+                                         '' if self.drought is None else ', drought={!r}'.format(self.drought)))
+
+
+def merge_drought_counts(a, na, b, nb):
+    """Drought count partial `a` (of na members) absorbs partial `b` (of nb members), in place; returns a.  The counts
+    are integers, so the sum is exact in any order."""
+    a[0].add_(b[0])
+    return a
 
 
 QUANTILE_CHUNK_BYTES = 2 << 30    # budget of the [n_members, chunk, ld] buffers that bring the members of several
@@ -234,6 +328,12 @@ class EnsembleRunner:
             self._reduce_vars = self.output_vars + (('q',) if spec.group_sums and 'q' not in self.output_vars else ())
         self._stats_state, self.n_stats = None, 0   # across-member accumulators: var -> (sum, m2) and (min, max)
         self._stack, self.n_stacked = None, 0       # quantiles: var -> every member's reduced field [n, ntime, ld]
+        self._drought = spec.drought if spec is not None else None
+        self._drought_count, self.n_drought = None, 0   # members in drought per month and cell, int32 [nmonths, ld]
+        if self._drought is not None:
+            self._drought.validate(statics.ncell, statics.start_yr, statics.end_yr)
+            self._drought_th = (None if self._drought.thresholds is None
+                                else torch.from_numpy(self._drought.thresholds).cuda())
         # One pair of copy streams per process and device, not per runner: torch's caching allocator keeps freed blocks
         # per STREAM, so every new stream starts with an empty pool - a runner per run_ensemble call with fresh streams
         # left 6 - 9 GB of staging blocks cached under dead streams per call, and after a dozen calls the allocator had
@@ -321,7 +421,9 @@ class EnsembleRunner:
         s, torch = self.s, self._torch
         compute = torch.cuda.current_stream()
         stream = self.front if self.front is not None else compute
-        want = tuple(k for k, v in (('aet', 'aet'), ('q', 'q'), ('sav', 'soilmoisture')) if v in self.output_vars or k == 'q')
+        dvar = self._drought.var if self._drought is not None else None
+        want = tuple(k for k, v in (('aet', 'aet'), ('q', 'q'), ('sav', 'soilmoisture'))
+                     if v in self.output_vars or k == 'q' or v == dvar)
         pets, ress = [], []
         with torch.cuda.stream(stream):
             while uploads:
@@ -366,10 +468,35 @@ class EnsembleRunner:
             results.append((out, agg))
         return results
 
+    def _drought_scan(self, out):
+        """The member's drought scan (compute stream) on its monthly mm field: its thresholds when the spec has none,
+        one xan_drought_scan that adds it to the counts and writes its summary (and its severity / intensity / duration
+        grids with spec.fields).  Returns the device tensors to copy back: {'summary': [4, ld], 'thresholds'?:
+        [nper, ncell], 'severity'? ...: cell-major [ncell, nmonths]}."""
+        from .drought.drought_stats import drought_scan_device, getthresh_device
+        d, s, torch = self._drought, self.s, self._torch
+        f = out[d.var]
+        if f.ld != s.ld:
+            raise RuntimeError("ensemble drought: field pitch {} differs from {}".format(f.ld, s.ld))
+        res = {'summary': torch.empty((len(DROUGHT_SUMMARY), s.ld), dtype=torch.float64, device='cuda')}
+        th = self._drought_th
+        if th is None:
+            first, end = d.reference_months(s.start_yr, s.end_yr)
+            th = res['thresholds'] = getthresh_device(f.t[first:end], s.ncell, d.nper)
+        sid = [C.Field.empty(s.ncell, s.nmonths, s.ld) for _ in DROUGHT_FIELDS] if d.fields else None
+        drought_scan_device(f.t, s.ncell, th, None if sid is None else [x.t for x in sid], self._drought_count,
+                            res['summary'])
+        self.n_drought += 1
+        for k, x in zip(DROUGHT_FIELDS, sid or ()):
+            res[k] = x.to_device_cell_major()
+        return res
+
     def _reduce(self, out):
         """The member's outputs as the spec asks for them (compute stream): yearly aggregation, km3, group sums of q,
-        and the member added to the across-member statistics.  Returns ({var: Field [ntime][ld]}, {scale: [ng, ntime]})."""
+        the member added to the across-member statistics and its drought scan.  Returns ({var: Field [ntime][ld]},
+        {scale: [ng, ntime]}, drought tensors or None)."""
         s, spec, lib = self.s, self.spec, C.lib()
+        drought = self._drought_scan(out) if self._drought is not None else None
         red = {}
         for v in self._reduce_vars:
             f = out[v]
@@ -405,16 +532,16 @@ class EnsembleRunner:
                 self._stack[v][self.n_stacked].copy_(red[v].t[:self.ntime], non_blocking=True)
             self.n_stacked += 1
         if not spec.member_fields:
-            return {}, groups
-        return {v: red[v] for v in self.output_vars}, groups
+            return {}, groups, drought
+        return {v: red[v] for v in self.output_vars}, groups, drought
 
     def _download(self, out, agg):
         torch = self._torch
         compute = torch.cuda.current_stream()
         if self.spec is None:
-            fields, groups = {v: out[v] for v in self.output_vars}, {}
+            fields, groups, drought = {v: out[v] for v in self.output_vars}, {}, None
         else:
-            fields, groups = self._reduce(out)
+            fields, groups, drought = self._reduce(out)
         staged = {v: f.to_device_cell_major() for v, f in fields.items()}      # transposes run on the compute stream
         ev = torch.cuda.Event()
         ev.record(compute)
@@ -440,6 +567,15 @@ class EnsembleRunner:
                     h = torch.empty(tuple(t.shape), dtype=torch.float64, pin_memory=True)
                     h.copy_(t, non_blocking=True)
                     host['group_sums'][g] = h
+                    self.d2h_bytes += h.numel() * 8
+            if drought is not None:     # summary and thresholds to pinned tensors, the grids through host_pool
+                host['drought'] = {}
+                for k, t in drought.items():
+                    t.record_stream(self.d2h)
+                    h = (C.host_pool.acquire(tuple(t.shape)) if k in DROUGHT_FIELDS
+                         else torch.empty(tuple(t.shape), dtype=torch.float64, pin_memory=True))
+                    h.copy_(t, non_blocking=True)
+                    host['drought'][k] = h[:, :self.s.ncell] if k == 'summary' else h
                     self.d2h_bytes += h.numel() * 8
             done = torch.cuda.Event(enable_timing=self.timeline is not None)
             done.record(self.d2h)
@@ -567,14 +703,30 @@ class EnsembleRunner:
         return self._quantiles(n, self._assembled(
             n, lambda v, t0, t1, buf: sharding.gather_rows_to_rank0(local(v, t0, t1), counts, buf)))
 
+    # ---- across-member drought frequency ----------------------------------------------------------------------------
+    def drought_partial(self):
+        """[int32 device tensor [nmonths, ld]]: members of the last `run` in drought per month and cell (None without
+        drought or before any member) - what `merge_drought_counts` combines and `finalize_drought` reports."""
+        if self._drought_count is None or self.n_drought == 0:
+            return None
+        return [self._drought_count]
+
+    def finalize_drought(self, partial, n):
+        """{'members_in_drought': int32 [ncell, nmonths], 'frequency': members_in_drought / n, 'n_members': n}."""
+        cnt = partial[0][:, :self.s.ncell].t().contiguous().cpu().numpy()
+        self.d2h_bytes += cnt.nbytes
+        return {'members_in_drought': cnt, 'frequency': cnt / n, 'n_members': int(n)}
+
     # ---- driver ----------------------------------------------------------------------------------------------------------
     def run(self, members):
         """Generator: yields (index, {variable: host ndarray [ncell, nmonths], 'basin_aggregates': [2, nmonths, n_basins]})
         in member order; the next members are being uploaded and a group of `group` members computed while the outputs of
         the group before are handed out.  With a spec the grids are [ncell, ntime] (none without member_fields), the
         result has 'group_sums': {scale: [ngroups, ntime]}, and each member is added to the across-member statistics
-        (`stats_partial` / `finalize_stats` once the generator is exhausted) and its reduced fields kept on the device for
-        the quantiles (`member_stack` / `finalize_quantiles`)."""
+        (`stats_partial` / `finalize_stats` once the generator is exhausted), its reduced fields kept on the device for
+        the quantiles (`member_stack` / `finalize_quantiles`), and with spec.drought the result has 'drought':
+        {'summary': {name: [ncell]}, 'thresholds'?: [nper, ncell], 'severity' / 'intensity' / 'duration'?:
+        [ncell, nmonths]} and the member is added to the drought counts (`drought_partial` / `finalize_drought`)."""
         torch = self._torch
         members = list(members)
         if not members:
@@ -583,9 +735,19 @@ class EnsembleRunner:
         n, depth, g = len(members), self.prefetch_depth, self.group
         # pinned output buffers in flight: the group being computed, the group before it on its way to the host, and the
         # results the caller still holds from the last hand-out - allocated before the pipeline starts, not inside it
+        in_flight, grids = min(3 * g, n + g), {}          # cells x time steps -> pinned grids the pipeline holds
         if self.spec is None or self.spec.member_fields:
-            C.host_pool.reserve((self.s.ncell, self.ntime), min(3 * g, n + g) * len(self.output_vars))
-        self.n_stats = self.n_stacked = 0
+            grids[self.ntime] = in_flight * len(self.output_vars)
+        if self._drought is not None and self._drought.fields:
+            grids[self.s.nmonths] = grids.get(self.s.nmonths, 0) + in_flight * len(DROUGHT_FIELDS)
+        for nt, count in grids.items():
+            C.host_pool.reserve((self.s.ncell, nt), count)
+        self.n_stats = self.n_stacked = self.n_drought = 0
+        if self._drought is not None:      # 4 B per month and cell, made before the pipeline starts
+            if self._drought_count is None:
+                self._drought_count = torch.zeros((self.s.nmonths, self.s.ld), dtype=torch.int32, device='cuda')
+            else:
+                self._drought_count.zero_()
         if self.spec is not None and self.spec.quantiles:
             self._alloc_stack(n)
         if self.spec is not None and self.spec.stats and self._stats_state is None:
@@ -645,6 +807,9 @@ class EnsembleRunner:
         for v, h in host.items():
             if v == 'group_sums':
                 res[v] = {g: t.numpy() for g, t in h.items()}
+            elif v == 'drought':
+                res[v] = {k: (dict(zip(DROUGHT_SUMMARY, t.numpy())) if k == 'summary'
+                              else C.host_pool.as_array(t) if k in DROUGHT_FIELDS else t.numpy()) for k, t in h.items()}
             else:
                 res[v] = C.host_pool.as_array(h) if v != 'basin_aggregates' else h.numpy()
         return k, res
@@ -676,6 +841,13 @@ def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=Tr
     before the run; at most 256 members.  Rank 0 gathers the members of all ranks point to point in rank order, a
     chunk of time steps at a time, and selects over them: the quantiles do not depend on the member order, so they
     are bitwise the same for every number of ranks.
+
+    With spec.drought every member's result has 'drought' (see EnsembleRunner.run), the returned dict has
+    'drought_summary': [n_members, 4, ncell] (DROUGHT_SUMMARY: drought months, events, longest duration, peak severity)
+    of all members in member order on every rank, and rank 0 gets 'ensemble_drought': {'members_in_drought': int32
+    [ncell, nmonths], 'frequency': members_in_drought / N, 'n_members': N}.  Each rank counts its members on the device
+    (int32 [nmonths, ld], 278 MB at 67,420 cells x 1,032 months) and rank 0 adds the counts of the other ranks: integer
+    sums are exact, so the counts and the frequency are bitwise the same for every number of ranks.
     """
     torch = C.torch_cuda()
     import torch.distributed as dist
@@ -692,11 +864,15 @@ def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=Tr
     groups = spec.group_sums if spec is not None else ()
     grp_local = {g: torch.zeros((len(mine), statics.group_table(g)[2], runner.ntime), dtype=torch.float64)
                  for g in groups}
+    drought = spec is not None and spec.drought is not None
+    dr_local = torch.zeros((len(mine), len(DROUGHT_SUMMARY), statics.ncell), dtype=torch.float64) if drought else None
     for j, res in runner.run([members[i] for i in mine]):
         if aggregates:
             agg_local[j] = torch.from_numpy(res['basin_aggregates'])
         for g in groups:
             grp_local[g][j] = torch.from_numpy(res['group_sums'][g])
+        if drought:
+            dr_local[j] = torch.from_numpy(np.stack([res['drought']['summary'][k] for k in DROUGHT_SUMMARY]))
         if on_result is not None:
             on_result(mine[j], res)
         else:
@@ -706,6 +882,12 @@ def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=Tr
     if groups:
         results['group_sums'] = {g: sharding.gather_ragged_rows(mine, grp_local[g].cuda(), len(members)).cpu().numpy()
                                  for g in groups}
+    if drought:
+        results['drought_summary'] = sharding.gather_ragged_rows(mine, dr_local.cuda(), len(members)).cpu().numpy()
+    if drought and members:
+        partial = sharding.fold_to_rank0(runner.drought_partial(), [len(p) for p in parts], merge_drought_counts)
+        if rank == 0:
+            results['ensemble_drought'] = runner.finalize_drought(partial, len(members))
     if spec is not None and spec.stats and members:
         partial = sharding.fold_to_rank0(runner.stats_partial(), [len(p) for p in parts], runner.merge_stats)
         if rank == 0:

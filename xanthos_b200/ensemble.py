@@ -24,6 +24,11 @@ data_writer/out_writer.py:60-110).  With torch.distributed initialised the membe
 An `OutputSpec` applies the reference's output options (yearly, km3, basin / country / region sums) and across-member
 statistics on the device, in front of the copy back (`run_ensemble(..., spec=...)`): the copy back, not the compute, is
 what limits multi-GPU runs, and a user who wants reduced output no longer pulls every monthly grid to the host.
+
+The PET model and the routing are those of the reference's [PET] and [Routing] sections: `EnsembleStatics(pet=...)`
+takes 'pm' (above), 'hs' (Hargreaves-Samani), 'thornthwaite' or 'none' (PET given with every member), and
+`routing=False` stops after ABCD: each member is then uploaded, run through PET -> ABCD and copied back on its own, and
+the run is bounded by the host -> device link.
 """
 
 from types import SimpleNamespace
@@ -32,18 +37,34 @@ import numpy as np
 
 from . import _cuda as C
 from . import sharding
+from .pet import hargreaves_samani as hs_mod
 from .pet import penman_monteith as pm_mod
+from .pet import thornthwaite as th_mod
 from .runoff import abcd as abcd_mod
 from .routing import mrtm as mrtm_mod
 
 PM_FORCING = ('tair_load', 'TMIN_load', 'rhs_load', 'wind_load', 'rsds_load', 'rlds_load')
 FORCING = PM_FORCING + ('precip', 'tmin')
+# the member fields of the PET models (pet_module of the .ini), named as DataLoader names them; ABCD adds precip, tmin
+PET_FORCING = {'pm': PM_FORCING, 'hs': ('hs_tas', 'hs_tmax', 'hs_tmin'), 'thornthwaite': ('tair',), 'none': ('pet',)}
+PET_MODELS = tuple(PET_FORCING)
 OUTPUTS = ('pet', 'aet', 'q', 'soilmoisture', 'chstorage', 'avgchflow')
+ROUTED_OUTPUTS = ('chstorage', 'avgchflow')
+PM_STATICS = ('pm_tables', 'lct_load', 'elev', 'water_idx', 'snow_idx', 'lc_years', 'nlcs')
+ROUTING_STATICS = ('flow_dist', 'velocity', 'upstream_matrix', 'ndays')
 GROUP_SCALES = ('basin', 'country', 'region')
 STATS = ('mean', 'std', 'min', 'max')
 DROUGHT_VARS = ('q', 'soilmoisture')
 DROUGHT_SUMMARY = ('drought_months', 'events', 'longest_duration', 'peak_severity')
 DROUGHT_FIELDS = ('severity', 'intensity', 'duration')
+
+
+def forcing_fields(pet):
+    """The keys of an ensemble member for PET model `pet` ('pm', 'hs', 'thornthwaite' or 'none'): the PET model's
+    fields, then 'precip' and 'tmin' of ABCD."""
+    if pet not in PET_FORCING:
+        raise C.ValidationException("unknown PET model {!r}; choose from {}".format(pet, PET_MODELS))
+    return PET_FORCING[pet] + ('precip', 'tmin')
 
 
 class DroughtSpec:
@@ -229,48 +250,93 @@ def lossless_float32(member, pin=True):
     on disk (NetCDF float variables) and only widened to float64 by the loader (data_load.py:288-340), so the copy is
     lossless: float -> double on the device is exact and every result stays bit-identical, while the host -> device
     traffic - the limiter of multi-GPU ensemble runs - halves.  NaN (missing data) counts as representable.
-    Call it once per member where the data are loaded; it costs a pass over the arrays on the host.
+    Call it once per member where the data are loaded; it costs a pass over the arrays on the host.  The forcing keys
+    of every PET model are converted (those the member has); an array that is several fields of the member (tmin
+    and hs_tmin read from one file) is converted once and stays one array, so it still crosses the link once.
     """
-    out = dict(member)
-    for k in FORCING:
-        a = np.asarray(member[k])
-        if a.dtype != np.float64:
+    out, done = dict(member), {}
+    for k in dict.fromkeys(key for pet in PET_MODELS for key in forcing_fields(pet)):
+        if k not in member:
             continue
-        a32 = a.astype(np.float32)
-        back = a32.astype(np.float64)
-        if np.array_equal(back, a, equal_nan=True):
-            if pin and C.device_available():
-                t = C.torch_cuda().from_numpy(a32).pin_memory()
-                a32 = t.numpy()
-            out[k] = a32
+        if id(member[k]) in done:
+            out[k] = done[id(member[k])]
+            continue
+        a = np.asarray(member[k])
+        if a.dtype == np.float64:
+            a32 = a.astype(np.float32)
+            back = a32.astype(np.float64)
+            if np.array_equal(back, a, equal_nan=True):
+                if pin and C.device_available():
+                    t = C.torch_cuda().from_numpy(a32).pin_memory()
+                    a32 = t.numpy()
+                out[k] = a32
+        done[id(member[k])] = out[k]
     return out
 
 
 class EnsembleStatics:
-    """Everything that does not change from member to member, staged on the device once."""
+    """
+    Everything that does not change from member to member, staged on the device once.
+
+      pet        PET model of the members, spelled as pet_module of the .ini: 'pm' (Penman-Monteith: pm_tables,
+                 lct_load, elev, water_idx, snow_idx, lc_years and nlcs are required), 'hs' (Hargreaves-Samani),
+                 'thornthwaite' or 'none' (every member brings its PET); other than 'pm' the PM arguments may be None
+                 and are not staged.  `forcing_fields(pet)` names the member keys.
+      latitude   degrees per cell (coords[:, 2]), required for 'hs' and 'thornthwaite' (in radians,
+                 np.radians(latitude), as DataLoader.lat_radians)
+      routing    False: no MRTM, the members stop after ABCD; flow_dist, velocity, upstream_matrix and ndays may be
+                 None and dt / routing_spinup are not used
+
+    A configuration that cannot run raises ValidationException here, naming what is missing.
+    """
 
     def __init__(self, ncell, start_yr, end_yr, pm_tables, lct_load, elev, water_idx, snow_idx, lc_years, nlcs,
                  n_basins, basin_ids, abcd_pars, area, flow_dist, velocity, upstream_matrix, ndays, dt=3 * 3600,
-                 runoff_spinup=None, routing_spinup=None, country_ids=None, region_ids=None):
+                 runoff_spinup=None, routing_spinup=None, country_ids=None, region_ids=None, pet='pm', latitude=None,
+                 routing=True):
+        forcing_fields(pet)
+        given = dict(zip(PM_STATICS + ROUTING_STATICS, (pm_tables, lct_load, elev, water_idx, snow_idx, lc_years, nlcs,
+                                                        flow_dist, velocity, upstream_matrix, ndays)))
+        need = (PM_STATICS if pet == 'pm' else ()) + (ROUTING_STATICS if routing else ())
+        missing = [k for k in need if given[k] is None]
+        if pet in ('hs', 'thornthwaite') and latitude is None:
+            missing.append('latitude')
+        if missing:
+            raise C.ValidationException("EnsembleStatics(pet={!r}, routing={}) needs {}".format(
+                pet, bool(routing), ', '.join(missing)))
+        if latitude is not None and np.asarray(latitude).reshape(-1).shape[0] != int(ncell):
+            raise C.ValidationException("latitude has {} entries for {} cells".format(
+                np.asarray(latitude).reshape(-1).shape[0], int(ncell)))
         torch = C.torch_cuda()
+        self.pet, self.routing = pet, bool(routing)
         self.ncell, self.start_yr, self.end_yr = int(ncell), int(start_yr), int(end_yr)
         self.nmonths = (self.end_yr - self.start_yr + 1) * 12
         self.ld = C.padded_ld(self.ncell)
-        self.tables = dict(pm_tables)
-        self.water_idx, self.snow_idx, self.lc_years, self.nlcs = int(water_idx), int(snow_idx), list(lc_years), int(nlcs)
-        self.d_lct = pm_mod.stage_land_cover(lct_load, self.ld)
-        self.d_elev = C.dev_vector(elev)
+        if pet == 'pm':
+            self.tables = dict(pm_tables)
+            self.water_idx, self.snow_idx = int(water_idx), int(snow_idx)
+            self.lc_years, self.nlcs = list(lc_years), int(nlcs)
+            self.d_lct = pm_mod.stage_land_cover(lct_load, self.ld)
+            self.d_elev = C.dev_vector(elev)
+        # HS takes degrees, Thornthwaite radians: np.radians of the float64 degrees, DataLoader's lat_radians bit for bit
+        self.d_lat = None
+        if pet in ('hs', 'thornthwaite'):
+            lat = np.asarray(latitude, dtype=np.float64).reshape(-1)
+            self.d_lat = C.dev_vector(lat if pet == 'hs' else np.radians(lat))
         self.n_basins = int(n_basins)
         self.basin_ids = np.asarray(basin_ids)
         rows = abcd_mod._basin_rows(self.n_basins, self.basin_ids, np.asarray(abcd_pars).shape[0])
         self.plan = abcd_mod.basin_plan(rows, self.n_basins)
         self.d_pars = torch.from_numpy(np.ascontiguousarray(abcd_pars, dtype=np.float64)).cuda()
-        self.d_area, self.d_L, self.d_V = C.dev_vector(area), C.dev_vector(flow_dist), C.dev_vector(velocity)
+        self.d_area = C.dev_vector(area)
         self.d_area_km3 = self.d_area * 1e-6
-        self.um = upstream_matrix
-        self.ndays = np.asarray(ndays, dtype=np.int32)[:self.nmonths]
-        self.dt = float(dt)
         self.runoff_spinup = self.nmonths if runoff_spinup is None else int(runoff_spinup)
+        self.d_L = self.d_V = self.um = self.ndays = None
+        if self.routing:
+            self.d_L, self.d_V = C.dev_vector(flow_dist), C.dev_vector(velocity)
+            self.um = upstream_matrix
+            self.ndays = np.asarray(ndays, dtype=np.int32)[:self.nmonths]
+        self.dt = float(dt)
         self.routing_spinup = self.nmonths if routing_spinup is None else int(routing_spinup)
         self.area = area
         self.group_ids = {'basin': self.basin_ids, 'country': country_ids, 'region': region_ids}
@@ -310,14 +376,22 @@ class EnsembleStatics:
 
 
 class EnsembleRunner:
-    def __init__(self, statics, output_vars=('q', 'avgchflow'), aggregates=True, prefetch_depth=4, group=2, spec=None):
+    def __init__(self, statics, output_vars=('q', 'avgchflow'), aggregates=True, prefetch_depth=4, group=None,
+                 spec=None):
         torch = C.torch_cuda()
         self.prefetch_depth = max(1, int(prefetch_depth))   # members whose forcing may be on its way ahead of the compute
-        self.group = max(1, int(group))                     # members routed by one launch
+        if group is None:                                   # members routed by one launch; nothing to share unrouted
+            group = 2 if statics.routing else 1
+        self.group = max(1, int(group))
         bad = [v for v in output_vars if v not in OUTPUTS]
         if bad:
             raise C.ValidationException("unknown output variable(s) {}; choose from {}".format(bad, OUTPUTS))
+        routed = [v for v in output_vars if v in ROUTED_OUTPUTS]
+        if routed and not statics.routing:
+            raise C.ValidationException("output variable(s) {} need routing; the statics have routing=False".format(
+                routed))
         self.s, self.output_vars, self.aggregates = statics, tuple(output_vars), bool(aggregates)
+        self.n_agg_rows = 2 if statics.routing else 1       # basin runoff (and the basin sum of the mean streamflow)
         self.spec = spec
         self.ntime = statics.nmonths // 12 if spec is not None and spec.output_in_year else statics.nmonths
         if spec is not None:
@@ -363,17 +437,26 @@ class EnsembleRunner:
         torch = self._torch
         if callable(member):
             member = member()
-        missing = [k for k in FORCING if k not in member]
+        keys = forcing_fields(self.s.pet)
+        missing = [k for k in keys if k not in member]
         if missing:
-            raise C.ValidationException("ensemble member lacks {}".format(missing))
+            raise C.ValidationException("ensemble member lacks {} (pet={!r})".format(missing, self.s.pet))
+        # an array that is several fields of the member (hs_tmin and tmin from one file) crosses the link once
+        first = {}
+        for k in keys:
+            first.setdefault(id(member[k]), k)
         staged = {}
-        bufs = {k: self._slot_buffer(slot, k) for k in FORCING}      # allocated on the compute stream (its pool is reused)
+        # staging buffers allocated on the compute stream (its pool is reused)
+        bufs = {k: self._slot_buffer(slot, k) for k in keys if first[id(member[k])] == k}
         # Only copy-engine work goes on the h2d stream.  The transposes to month-major run on the compute stream in front
         # of the member's kernels: a kernel on the h2d stream would wait for SM resources behind the routing kernel of
         # the previous member (one cooperative block per SM, the whole register file) and hold up the next copy.
         with torch.cuda.stream(self.h2d):
             e0 = self._mark(self.h2d)
-            for k in FORCING:
+            for k in keys:
+                if first[id(member[k])] != k:
+                    staged[k] = staged[first[id(member[k])]]
+                    continue
                 a = member[k]
                 if tuple(a.shape) != (self.s.ncell, self.s.nmonths):
                     raise C.ValidationException("member field {} has shape {}, expected {}".format(
@@ -399,12 +482,15 @@ class EnsembleRunner:
         return staged, ev
 
     def _to_fields(self, staged):
-        """cell-major staging tensors -> month-major Fields (compute stream)."""
+        """cell-major staging tensors -> month-major Fields (compute stream).  Outside PM, ABCD's tmin is read with NaN
+        as 0 (DataLoader loads TempMinFile with nan_to_num; idempotent on an array it cleaned already), while HS reads
+        hs_tmin - possibly the same upload - as it is."""
         fields = {}
         for k, t in staged.items():
             f = C.Field.empty(self.s.ncell, self.s.nmonths, self.s.ld)
             fn = C.lib().xan_to_month_major_f32 if t.dtype == self._torch.float32 else C.lib().xan_to_month_major
-            C.check(fn(C.ptr(t), C.ptr(f.t), self.s.ncell, self.s.nmonths, f.ld, 0, C.stream_ptr()))
+            nan_to_num = int(k == 'tmin' and self.s.pet != 'pm')
+            C.check(fn(C.ptr(t), C.ptr(f.t), self.s.ncell, self.s.nmonths, f.ld, nan_to_num, C.stream_ptr()))
             fields[k] = f
         return fields
 
@@ -415,8 +501,20 @@ class EnsembleRunner:
         e.record(stream)
         return e
 
+    def _pet(self, fields):
+        """The member's PET Field from its month-major forcing (current stream)."""
+        s = self.s
+        if s.pet == 'pm':
+            return pm_mod.run_pmpet_device(s.data_ns(fields), s.ncell, s.nlcs, s.start_yr, s.end_yr, s.water_idx,
+                                           s.snow_idx, s.lc_years)
+        if s.pet == 'hs':
+            return hs_mod.execute_device(fields['hs_tas'], fields['hs_tmax'], fields['hs_tmin'], s.d_lat, s.start_yr)
+        if s.pet == 'thornthwaite':
+            return th_mod.execute_device(fields['tair'], s.d_lat, s.start_yr)
+        return fields['pet']
+
     def _front(self, uploads):
-        """Front stage, per member: wait for its upload, transposes, PM -> ABCD.  `uploads`: [(staged tensors, upload event)].
+        """Front stage, per member: wait for its upload, transposes, PET -> ABCD.  `uploads`: [(staged tensors, upload event)].
         Runs on the front stream (beside the routing launch of the group before); returns (PET Fields, ABCD results, event)."""
         s, torch = self.s, self._torch
         compute = torch.cuda.current_stream()
@@ -431,8 +529,7 @@ class EnsembleRunner:
                 stream.wait_event(ev)     # the first member's PET and runoff run under the second member's upload
                 fields = self._to_fields(staged)
                 del staged
-                pet = pm_mod.run_pmpet_device(s.data_ns(fields), s.ncell, s.nlcs, s.start_yr, s.end_yr, s.water_idx,
-                                              s.snow_idx, s.lc_years)
+                pet = self._pet(fields)
                 res = abcd_mod.run_device(s.plan, s.d_pars, pet, fields['precip'], fields['tmin'], s.nmonths,
                                           s.runoff_spinup, want=want)
                 if stream is not compute:     # allocated on the front stream, read by the routing / output stage
@@ -445,10 +542,12 @@ class EnsembleRunner:
         return pets, ress, ev
 
     def _back(self, pets, ress):
-        """One routing call for the group and the basin aggregates per member (compute stream)."""
+        """One routing call for the group (with routing) and the basin aggregates per member (compute stream)."""
         s = self.s
         want_chs = 'chstorage' in self.output_vars
-        if len(ress) == 1:
+        if not s.routing:
+            routed = [(None, None, None)] * len(ress)
+        elif len(ress) == 1:
             routed = [mrtm_mod.route_device(s.um, ress[0]['q'], s.d_L, s.d_V, s.d_area, s.ndays, s.dt, s.routing_spinup,
                                             want_chs=want_chs)]
         else:
@@ -460,11 +559,13 @@ class EnsembleRunner:
                    'avgchflow': avg}
             agg = None
             if self.aggregates:   # basin runoff in km3 / month and basin sum of the mean streamflow, [2, nmonths, n_basins]
-                agg = self._torch.empty((2, s.nmonths, s.n_basins), dtype=self._torch.float64, device='cuda')
+                agg = self._torch.empty((self.n_agg_rows, s.nmonths, s.n_basins), dtype=self._torch.float64,
+                                        device='cuda')
                 C.check(C.lib().xan_basin_sum(s.plan._plan, C.ptr(res['q'].t), C.ptr(s.d_area_km3), s.nmonths,
                                               res['q'].ld, C.ptr(agg[0]), C.stream_ptr()))
-                C.check(C.lib().xan_basin_sum(s.plan._plan, C.ptr(avg.t), None, s.nmonths, avg.ld, C.ptr(agg[1]),
-                                              C.stream_ptr()))
+                if s.routing:     # without routing [1, nmonths, n_basins]: the runoff row only
+                    C.check(C.lib().xan_basin_sum(s.plan._plan, C.ptr(avg.t), None, s.nmonths, avg.ld, C.ptr(agg[1]),
+                                                  C.stream_ptr()))
             results.append((out, agg))
         return results
 
@@ -719,9 +820,9 @@ class EnsembleRunner:
 
     # ---- driver ----------------------------------------------------------------------------------------------------------
     def run(self, members):
-        """Generator: yields (index, {variable: host ndarray [ncell, nmonths], 'basin_aggregates': [2, nmonths, n_basins]})
-        in member order; the next members are being uploaded and a group of `group` members computed while the outputs of
-        the group before are handed out.  With a spec the grids are [ncell, ntime] (none without member_fields), the
+        """Generator: yields (index, {variable: host ndarray [ncell, nmonths], 'basin_aggregates': [n_agg_rows, nmonths,
+        n_basins]}) in member order; the next members are being uploaded and a group of `group` members computed while
+        the outputs of the group before are handed out.  With a spec the grids are [ncell, ntime] (none without member_fields), the
         result has 'group_sums': {scale: [ngroups, ntime]}, and each member is added to the across-member statistics
         (`stats_partial` / `finalize_stats` once the generator is exhausted), its reduced fields kept on the device for
         the quantiles (`member_stack` / `finalize_quantiles`), and with spec.drought the result has 'drought':
@@ -821,7 +922,8 @@ def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=Tr
     sharding.partition_members).
     Returns {member index: result dict}; with `on_result(index, result)` given the results are handed to it instead of
     being kept (a 64-member ensemble of 1,032 months is 2 x 36 GB of output).  On every rank the returned dict also has
-    the key 'basin_aggregates': [n_members, 2, nmonths, n_basins] of ALL members (all-gather over NCCL).
+    the key 'basin_aggregates': [n_members, 2, nmonths, n_basins] of ALL members (all-gather over NCCL); without
+    routing (EnsembleStatics(routing=False)) it is [n_members, 1, nmonths, n_basins], the basin runoff in km3 / month.
 
     `spec` (OutputSpec) reduces the outputs on the device before they are copied back; without it every member's
     monthly grids come back as they are.  With it:
@@ -860,7 +962,7 @@ def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=Tr
     mine = [int(i) for i in parts[rank]]
     runner = EnsembleRunner(statics, output_vars, aggregates, spec=spec)
     results = {}
-    agg_local = torch.zeros((len(mine), 2, statics.nmonths, statics.n_basins), dtype=torch.float64)
+    agg_local = torch.zeros((len(mine), runner.n_agg_rows, statics.nmonths, statics.n_basins), dtype=torch.float64)
     groups = spec.group_sums if spec is not None else ()
     grp_local = {g: torch.zeros((len(mine), statics.group_table(g)[2], runner.ntime), dtype=torch.float64)
                  for g in groups}

@@ -113,6 +113,16 @@ int xan_abcd_run(const xan_abcd_plan *plan, const double *d_pet, const double *d
                  const double *d_tmin, const double *d_pars, int nmonths, int spinup, int ld,
                  double *d_aet, double *d_q, double *d_sav, void *stream);
 
+/* n_sets parameter tables over the same forcing in one call.  d_pars: [n_sets][n_rows][5], n_rows = the rows of
+ * ONE table (its stride; the rows the plan maps live cells to must be < n_rows, as for xan_abcd_run).
+ * h_aet / h_q / h_sav: HOST arrays of n_sets DEVICE pointers; the arrays and any entry may be NULL.
+ * Set s is bit-identical to xan_abcd_run(plan, ..., d_pars + s * n_rows * 5, ...).  1 <= n_sets <= XAN_ABCD_MAX_SETS. */
+#define XAN_ABCD_MAX_SETS 8
+int xan_abcd_run_sets(const xan_abcd_plan *plan, int n_sets, int n_rows, const double *d_pet,
+                      const double *d_precip, const double *d_tmin, const double *d_pars, int nmonths,
+                      int spinup, int ld, double *const *h_aet, double *const *h_q, double *const *h_sav,
+                      void *stream);
+
 /* Calibration objective for a batch of parameter sets; replaces objective_kge + basin_runoff
  * (xanthos/calibrate/calibrate_abcd.py:134-162, 176-213) evaluated `npar` times per basin.
  * For basin b = h_basins[i] (row of the plan) and parameter set p:

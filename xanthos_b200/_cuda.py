@@ -22,6 +22,7 @@ MRTM_AUTO, MRTM_GRID, MRTM_TREE, MRTM_SKEW = 0, 1, 2, 3
 PM_MAX_CLASSES = 32
 ENS_MAX_MEMBERS, ENS_MAX_LEVELS = 256, 64      # XAN_ENS_MAX_MEMBERS / XAN_ENS_MAX_LEVELS (xan_ens_quantiles)
 DROUGHT_MAX_YEARS = 1024                        # MAX_YEARS of xan_drought_thresholds: samples per (period, cell)
+ABCD_MAX_SETS = 8                               # XAN_ABCD_MAX_SETS: parameter tables per xan_abcd_run_sets call
 
 
 class ValidationException(Exception):
@@ -55,6 +56,8 @@ SIGNATURES = {
     'xan_abcd_plan_create': (_P, [POINTER(c_int), c_int, c_int]),
     'xan_abcd_plan_destroy': (None, [_P]),
     'xan_abcd_run': (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, _P, _P, _P, _P]),
+    'xan_abcd_run_sets': (c_int, [_P, c_int, c_int, _P, _P, _P, _P, c_int, c_int, c_int, POINTER(_P), POINTER(_P),
+                                  POINTER(_P), _P]),
     'xan_abcd_kge_batch': (c_int, [_P, POINTER(c_int), c_int, c_int, _P, _P, _P, _P, _P, _P, c_int, c_int, c_int,
                                    c_int, _P, _P, _P]),
     'xan_mrtm_downstream': (c_int, [POINTER(c_double), POINTER(c_double), c_int, c_int, c_int, POINTER(c_int64)]),
@@ -99,7 +102,8 @@ _lib = None
 # kernels launched by each entry point (the claim behind bench.py's "gpu_launches")
 KERNELS_PER_CALL = {
     'xan_to_month_major': 1, 'xan_to_month_major_f32': 1, 'xan_to_cell_major': 1, 'xan_hs_pet': 2, 'xan_thornthwaite_pet': 2,
-    'xan_thornthwaite_daylight': 1, 'xan_pm_pet': 1, 'xan_abcd_run': 3, 'xan_abcd_kge_batch': 1,
+    'xan_thornthwaite_daylight': 1, 'xan_pm_pet': 1, 'xan_abcd_run': 3, 'xan_abcd_run_sets': 3,
+    'xan_abcd_kge_batch': 1,
     'xan_mrtm_route': 1, 'xan_mrtm_route_batch': 1, 'xan_hargreaves_pet': 1, 'xan_gwam_run': 1, 'xan_agg_to_year': 1, 'xan_basin_sum': 1,
     'xan_drought_stats': 1, 'xan_drought_scan': 1, 'xan_drought_thresholds': 1, 'xan_group_sum': 1, 'xan_year_sum_scaled': 1,
     'xan_scale_cells': 1, 'xan_ens_stats_update': 1, 'xan_ens_stats_merge': 1, 'xan_ens_stats_finalize': 1,

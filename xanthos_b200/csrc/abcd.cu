@@ -195,19 +195,55 @@ __device__ __forceinline__ void abcd_stream(const double *__restrict__ pet, cons
 }
 constexpr size_t ABCD_RING_BYTES = sizeof(double) * ABCD_STAGES * ABCD_SM * 3 * ABCD_BLOCK;   // 48 KB per block
 
+// Sets of parameter tables over one forcing (xan_abcd_run_sets): a thread steps K sets through every month it reads from
+// the ring, so each forcing value is read once per K sets, and the K recurrences are independent (instruction-level
+// parallelism in the latency-bound month chain).  blockIdx.y = group of K sets; the last group of a call may be short
+// (nk < K): its spare slots repeat the group's last set and write nothing.  xan_abcd_run is the K = 1 instance.
+// K = 2 (B200, tools/parameter_ensemble_bench.py, DESIGN.md section 6): 0.334 ms per set at 8 sets per call against
+// 0.405 with K = 1 and 0.525 for single-set calls; K = 4 spills under the 128-register budget of 4 blocks per SM.
+constexpr int ABCD_SETS_PER_THREAD = 2;
+static_assert(XAN_ABCD_MAX_SETS % ABCD_SETS_PER_THREAD == 0, "whole groups at the largest call");
+
+struct AbcdSetOut {   // device output pointers of every set, passed by value in the kernel parameters
+    double *aet[XAN_ABCD_MAX_SETS], *q[XAN_ABCD_MAX_SETS], *sav[XAN_ABCD_MAX_SETS];
+};
+
+// Parameters of the K sets of this thread; true when every divisor of every set is covered by the fast division.
+// A thread whose sets are not all covered takes the generic template, in which div_const decides per set: both give
+// the same bits, so a set's result does not depend on the sets it is grouped with.
+template <int K>
+__device__ __forceinline__ bool load_pars(const double *__restrict__ pars, int n_rows, int s0, int nk, int row,
+                                          bool snow, AbcdPar (&par)[K]) {
+    bool ok = true;
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        par[j] = load_par(pars + (size_t)(s0 + min(j, nk - 1)) * n_rows * 5, row, snow);
+        ok = ok && par[j].exact_ok;
+    }
+    return ok;
+}
+
 // 4 blocks of 128 threads per SM (<= 128 registers): 67,420 cells are 527 blocks = 3.6 per SM, one wave
-template <bool SNOW>
+template <bool SNOW, int K>
 __global__ void __launch_bounds__(128, 4)
     abcd_spinup_kernel(const double *__restrict__ pet, const double *__restrict__ precip,
                        const double *__restrict__ tmin, const int *__restrict__ basin_idx,
-                       const double *__restrict__ pars, int ncell, int spinup, int ld,
-                       double *__restrict__ snap /* [6][ncell]: SW x3, G x3 */) {
+                       const double *__restrict__ pars, int n_rows, int n_sets, int ncell, int spinup, int ld,
+                       double *__restrict__ snap /* [n_sets][6][ncell]: SW x3, G x3 */) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= ncell) return;
     const int row = basin_idx[c];
     if (row < 0) return;
-    const AbcdPar par = load_par(pars, row, SNOW);
-    double snowpack = 0.0, sw = SW_INIT, g = GW_INIT;
+    const int s0 = blockIdx.y * K, nk = min(K, n_sets - s0);
+    AbcdPar par[K];
+    const bool fast_all = load_pars<K>(pars, n_rows, s0, nk, row, SNOW, par);
+    double snowpack[K], sw[K], g[K];
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        snowpack[j] = 0.0;
+        sw[j] = SW_INIT;
+        g[j] = GW_INIT;
+    }
     const int s1 = spinup - 25, s2 = spinup - 13, s3 = spinup - 1;   // Decembers -25, -13, -1 (:255)
     // three segments ending at the three Decembers whose state is kept: no per-month test for the snapshot months
     auto run = [&](auto fast) {
@@ -216,15 +252,24 @@ __global__ void __launch_bounds__(128, 4)
         for (int seg = 0; seg < 3; ++seg) {
             const int last = seg == 0 ? s1 : (seg == 1 ? s2 : s3);
             abcd_stream<SNOW>(pet, precip, tmin, c, ld, last + 1, [&](int k, double p, double e, double t) {
-                double aet, q;
-                abcd_step<SNOW, decltype(fast)::value>(k == 0, p, e, t, par, snowpack, sw, g, aet, q);
+#pragma unroll
+                for (int j = 0; j < K; ++j) {
+                    double aet, q;
+                    abcd_step<SNOW, decltype(fast)::value>(k == 0, p, e, t, par[j], snowpack[j], sw[j], g[j], aet, q);
+                }
             }, begin);
-            snap[(2 - seg) * (size_t)ncell + c] = sw;
-            snap[(5 - seg) * (size_t)ncell + c] = g;
+#pragma unroll
+            for (int j = 0; j < K; ++j) {
+                if (j < nk) {
+                    double *sn = snap + (size_t)(s0 + j) * 6 * ncell;
+                    sn[(2 - seg) * (size_t)ncell + c] = sw[j];
+                    sn[(5 - seg) * (size_t)ncell + c] = g[j];
+                }
+            }
             begin = last + 1;
         }
     };
-    if (par.exact_ok) run(std::true_type{});      // practically always: no divisor with an all-ones significand
+    if (fast_all) run(std::true_type{});      // practically always: no divisor with an all-ones significand
     else run(std::false_type{});
 }
 
@@ -254,12 +299,14 @@ __device__ __forceinline__ void block_reduce2(double &s, double &n, double *scra
     }
 }
 
-// set_vals (abcd.py:246-282): per basin, mean over the 3 Decembers of nanmean over cells.
+// set_vals (abcd.py:246-282): per basin, mean over the 3 Decembers of nanmean over cells.  blockIdx.y = parameter set.
 __global__ void __launch_bounds__(256)
-    abcd_reinit_kernel(const double *__restrict__ snap, const int *__restrict__ order,
-                       const int *__restrict__ offsets, int ncell, double *__restrict__ init /* [nb][2] */) {
+    abcd_reinit_kernel(const double *__restrict__ snap /* [n_sets][6][ncell] */, const int *__restrict__ order,
+                       const int *__restrict__ offsets, int ncell, double *__restrict__ init /* [n_sets][nb][2] */) {
     __shared__ double scratch[16];
     const int b = blockIdx.x;
+    snap += (size_t)blockIdx.y * 6 * ncell;
+    init += (size_t)blockIdx.y * 2 * gridDim.x;
     const int beg = offsets[b], end = offsets[b + 1];
     double mean3[2];
     for (int v = 0; v < 2; ++v) {
@@ -285,39 +332,62 @@ __global__ void __launch_bounds__(256)
     }
 }
 
-template <bool SNOW>
+template <bool SNOW, int K>
 __global__ void __launch_bounds__(128, 4)
     abcd_sim_kernel(const double *__restrict__ pet, const double *__restrict__ precip,
                     const double *__restrict__ tmin, const int *__restrict__ basin_idx,
-                    const double *__restrict__ pars, const double *__restrict__ init, int ncell, int nmonths,
-                    int ld, double *__restrict__ aet_o, double *__restrict__ q_o, double *__restrict__ sav_o) {
+                    const double *__restrict__ pars, int n_rows, int n_sets,
+                    const double *__restrict__ init /* [n_sets][nb][2] */, int n_basins, int ncell, int nmonths,
+                    int ld, const AbcdSetOut out) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= ncell) return;
+    const int s0 = blockIdx.y * K, nk = min(K, n_sets - s0);
+    double *aet_o[K], *q_o[K], *sav_o[K];     // NULL: not requested, or a spare slot of a short group
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        aet_o[j] = j < nk ? out.aet[s0 + j] : nullptr;
+        q_o[j] = j < nk ? out.q[s0 + j] : nullptr;
+        sav_o[j] = j < nk ? out.sav[s0 + j] : nullptr;
+    }
     const int row = basin_idx[c];
     if (row < 0) {
         // not simulated: the reference leaves these rows uninitialised (abcd.py:384-389)
         const double nanv = __longlong_as_double(0x7ff8000000000000LL);
         for (int i = 0; i < nmonths; ++i) {
             const size_t off = (size_t)i * ld + c;
-            if (aet_o) aet_o[off] = nanv;
-            if (q_o) q_o[off] = nanv;
-            if (sav_o) sav_o[off] = nanv;
+#pragma unroll
+            for (int j = 0; j < K; ++j) {
+                if (aet_o[j]) aet_o[j][off] = nanv;
+                if (q_o[j]) q_o[j][off] = nanv;
+                if (sav_o[j]) sav_o[j][off] = nanv;
+            }
         }
         return;
     }
-    const AbcdPar par = load_par(pars, row, SNOW);
-    double snowpack = 0.0, sw = init[2 * row], g = init[2 * row + 1];
+    AbcdPar par[K];
+    const bool fast_all = load_pars<K>(pars, n_rows, s0, nk, row, SNOW, par);
+    double snowpack[K], sw[K], g[K];
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        const double *in = init + ((size_t)(s0 + min(j, nk - 1)) * n_basins + row) * 2;
+        snowpack[j] = 0.0;
+        sw[j] = in[0];
+        g[j] = in[1];
+    }
     auto run = [&](auto fast) {
         abcd_stream<SNOW>(pet, precip, tmin, c, ld, nmonths, [&](int k, double p, double e, double t) {
-            double aet, q;
-            abcd_step<SNOW, decltype(fast)::value>(k == 0, p, e, t, par, snowpack, sw, g, aet, q);
             const size_t off = (size_t)k * ld + c;
-            if (aet_o) stg_stream(aet_o + off, aet);
-            if (q_o) stg_stream(q_o + off, q);
-            if (sav_o) stg_stream(sav_o + off, sw);
+#pragma unroll
+            for (int j = 0; j < K; ++j) {
+                double aet, q;
+                abcd_step<SNOW, decltype(fast)::value>(k == 0, p, e, t, par[j], snowpack[j], sw[j], g[j], aet, q);
+                if (aet_o[j]) stg_stream(aet_o[j] + off, aet);
+                if (q_o[j]) stg_stream(q_o[j] + off, q);
+                if (sav_o[j]) stg_stream(sav_o[j] + off, sw[j]);
+            }
         });
     };
-    if (par.exact_ok) run(std::true_type{});
+    if (fast_all) run(std::true_type{});
     else run(std::false_type{});
 }
 
@@ -673,6 +743,60 @@ __global__ void __launch_bounds__(256)
 
 using namespace xan;
 
+// The three launches of n_sets tables, K sets per thread of the two passes.
+template <int K>
+static int abcd_launch(const xan_abcd_plan *pl, int n_sets, int n_rows, const double *d_pet, const double *d_precip,
+                       const double *d_tmin, const double *d_pars, int nmonths, int spinup, int ld,
+                       const AbcdSetOut &out, cudaStream_t s) {
+    const int ncell = pl->ncell;
+    double *snap = nullptr, *init = nullptr;
+    XAN_CUDA_CHECK(scratch_alloc(&snap, sizeof(double) * 6 * (size_t)ncell * n_sets, s));
+    XAN_CUDA_CHECK(scratch_alloc(&init, sizeof(double) * 2 * (size_t)pl->n_basins * n_sets, s));
+    const dim3 grid(ceil_div(ncell, ABCD_BLOCK), ceil_div(n_sets, K));
+    {   // 4 blocks x 48 KB of ring per SM: ask for the large shared-memory carve-out (otherwise the 527 blocks of the
+        // 0.5 degree grid do not fit in one wave)
+        static bool once = false;
+        if (!once) {
+            once = true;
+            cudaFuncSetAttribute(abcd_spinup_kernel<true, K>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+            cudaFuncSetAttribute(abcd_spinup_kernel<false, K>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+            cudaFuncSetAttribute(abcd_sim_kernel<true, K>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+            cudaFuncSetAttribute(abcd_sim_kernel<false, K>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        }
+    }
+    if (d_tmin)
+        abcd_spinup_kernel<true, K><<<grid, ABCD_BLOCK, ABCD_RING_BYTES, s>>>(d_pet, d_precip, d_tmin, pl->d_basin_idx,
+                                                                              d_pars, n_rows, n_sets, ncell, spinup, ld,
+                                                                              snap);
+    else
+        abcd_spinup_kernel<false, K><<<grid, ABCD_BLOCK, ABCD_RING_BYTES, s>>>(d_pet, d_precip, d_tmin, pl->d_basin_idx,
+                                                                               d_pars, n_rows, n_sets, ncell, spinup, ld,
+                                                                               snap);
+    abcd_reinit_kernel<<<dim3(pl->n_basins, n_sets), 256, 0, s>>>(snap, pl->d_order, pl->d_offsets, ncell, init);
+    if (d_tmin)
+        abcd_sim_kernel<true, K><<<grid, ABCD_BLOCK, ABCD_RING_BYTES, s>>>(d_pet, d_precip, d_tmin, pl->d_basin_idx,
+                                                                           d_pars, n_rows, n_sets, init, pl->n_basins,
+                                                                           ncell, nmonths, ld, out);
+    else
+        abcd_sim_kernel<false, K><<<grid, ABCD_BLOCK, ABCD_RING_BYTES, s>>>(d_pet, d_precip, d_tmin, pl->d_basin_idx,
+                                                                            d_pars, n_rows, n_sets, init, pl->n_basins,
+                                                                            ncell, nmonths, ld, out);
+    XAN_CUDA_CHECK(cudaGetLastError());
+    XAN_CUDA_CHECK(cudaFreeAsync(snap, s));
+    XAN_CUDA_CHECK(cudaFreeAsync(init, s));
+    return XAN_OK;
+}
+
+static int abcd_check_spinup(int spinup) {
+    if (spinup < 25) {
+        // ABCD.set_vals indexes month -25 of the spin-up arrays (abcd.py:255-266)
+        set_error("Spin-up steps must produce at least 10 years spin-up. Your spin-up only consist of %d months. "
+                  "Please reconfigure and try again.", spinup);
+        return XAN_E_SPINUP;
+    }
+    return XAN_OK;
+}
+
 extern "C" {
 
 xan_abcd_plan *xan_abcd_plan_create(const int *h_basin_idx, int ncell, int n_basins) {
@@ -733,47 +857,44 @@ int xan_abcd_run(const xan_abcd_plan *pl, const double *d_pet, const double *d_p
                  double *d_sav, void *stream) {
     XAN_REQUIRE(pl && d_pet && d_precip && d_pars, "xan_abcd_run: null pointer");
     XAN_REQUIRE(nmonths > 0 && ld >= pl->ncell, "xan_abcd_run: bad shape nmonths=%d ld=%d", nmonths, ld);
-    if (spinup < 25) {
-        // ABCD.set_vals indexes month -25 of the spin-up arrays (abcd.py:255-266)
-        set_error("Spin-up steps must produce at least 10 years spin-up. Your spin-up only consist of %d months. "
-                  "Please reconfigure and try again.", spinup);
-        return XAN_E_SPINUP;
-    }
+    if (abcd_check_spinup(spinup) != XAN_OK) return XAN_E_SPINUP;
     XAN_REQUIRE(spinup <= nmonths, "xan_abcd_run: spinup (%d) exceeds the %d months of forcing", spinup, nmonths);
-    cudaStream_t s = (cudaStream_t)stream;
-    const int ncell = pl->ncell;
-    double *snap = nullptr, *init = nullptr;
-    XAN_CUDA_CHECK(scratch_alloc(&snap, sizeof(double) * 6 * (size_t)ncell, s));
-    XAN_CUDA_CHECK(scratch_alloc(&init, sizeof(double) * 2 * (size_t)pl->n_basins, s));
-    const int grid = ceil_div(ncell, ABCD_BLOCK);
-    {   // 4 blocks x 48 KB of ring per SM: ask for the large shared-memory carve-out (otherwise the 527 blocks of the
-        // 0.5 degree grid do not fit in one wave)
-        static bool once = false;
-        if (!once) {
-            once = true;
-            cudaFuncSetAttribute(abcd_spinup_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-            cudaFuncSetAttribute(abcd_spinup_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-            cudaFuncSetAttribute(abcd_sim_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-            cudaFuncSetAttribute(abcd_sim_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-        }
+    AbcdSetOut out{};
+    out.aet[0] = d_aet;
+    out.q[0] = d_q;
+    out.sav[0] = d_sav;
+    return abcd_launch<1>(pl, 1, pl->n_basins, d_pet, d_precip, d_tmin, d_pars, nmonths, spinup, ld, out,
+                          (cudaStream_t)stream);
+}
+
+int xan_abcd_run_sets(const xan_abcd_plan *pl, int n_sets, int n_rows, const double *d_pet, const double *d_precip,
+                      const double *d_tmin, const double *d_pars, int nmonths, int spinup, int ld,
+                      double *const *h_aet, double *const *h_q, double *const *h_sav, void *stream) {
+    XAN_REQUIRE(pl && d_pet && d_precip && d_pars, "xan_abcd_run_sets: null pointer");
+    XAN_REQUIRE(n_sets >= 1 && n_sets <= XAN_ABCD_MAX_SETS, "xan_abcd_run_sets: n_sets=%d outside 1 .. %d", n_sets,
+                XAN_ABCD_MAX_SETS);
+    XAN_REQUIRE(n_rows >= 1, "xan_abcd_run_sets: n_rows=%d", n_rows);
+    XAN_REQUIRE(nmonths > 0 && ld >= pl->ncell, "xan_abcd_run_sets: bad shape nmonths=%d ld=%d", nmonths, ld);
+    if (abcd_check_spinup(spinup) != XAN_OK) return XAN_E_SPINUP;
+    XAN_REQUIRE(spinup <= nmonths, "xan_abcd_run_sets: spinup (%d) exceeds the %d months of forcing", spinup,
+                nmonths);
+    int max_row = -1;   // the last row the plan maps a live cell to: every table must have it
+    for (int b = 0; b < pl->n_basins; ++b)
+        if (pl->h_offsets[b + 1] > pl->h_offsets[b]) max_row = b;
+    XAN_REQUIRE(max_row < n_rows, "xan_abcd_run_sets: the plan maps cells to row %d, the tables have %d rows",
+                max_row, n_rows);
+    AbcdSetOut out{};
+    for (int k = 0; k < n_sets; ++k) {
+        out.aet[k] = h_aet ? h_aet[k] : nullptr;
+        out.q[k] = h_q ? h_q[k] : nullptr;
+        out.sav[k] = h_sav ? h_sav[k] : nullptr;
     }
-    if (d_tmin)
-        abcd_spinup_kernel<true><<<grid, ABCD_BLOCK, ABCD_RING_BYTES, s>>>(d_pet, d_precip, d_tmin, pl->d_basin_idx, d_pars, ncell,
-                                                      spinup, ld, snap);
-    else
-        abcd_spinup_kernel<false><<<grid, ABCD_BLOCK, ABCD_RING_BYTES, s>>>(d_pet, d_precip, d_tmin, pl->d_basin_idx, d_pars, ncell,
-                                                       spinup, ld, snap);
-    abcd_reinit_kernel<<<pl->n_basins, 256, 0, s>>>(snap, pl->d_order, pl->d_offsets, ncell, init);
-    if (d_tmin)
-        abcd_sim_kernel<true><<<grid, ABCD_BLOCK, ABCD_RING_BYTES, s>>>(d_pet, d_precip, d_tmin, pl->d_basin_idx, d_pars, init, ncell,
-                                                   nmonths, ld, d_aet, d_q, d_sav);
-    else
-        abcd_sim_kernel<false><<<grid, ABCD_BLOCK, ABCD_RING_BYTES, s>>>(d_pet, d_precip, d_tmin, pl->d_basin_idx, d_pars, init, ncell,
-                                                    nmonths, ld, d_aet, d_q, d_sav);
-    XAN_CUDA_CHECK(cudaGetLastError());
-    XAN_CUDA_CHECK(cudaFreeAsync(snap, s));
-    XAN_CUDA_CHECK(cudaFreeAsync(init, s));
-    return XAN_OK;
+    // one set alone takes the K = 1 instance: a group of K would step its spare slot through every month for nothing
+    if (n_sets == 1)
+        return abcd_launch<1>(pl, 1, n_rows, d_pet, d_precip, d_tmin, d_pars, nmonths, spinup, ld, out,
+                              (cudaStream_t)stream);
+    return abcd_launch<ABCD_SETS_PER_THREAD>(pl, n_sets, n_rows, d_pet, d_precip, d_tmin, d_pars, nmonths, spinup,
+                                             ld, out, (cudaStream_t)stream);
 }
 
 // Population layout of the calibration objective (see kge_pop_pass_kernel).

@@ -29,6 +29,10 @@ The PET model and the routing are those of the reference's [PET] and [Routing] s
 takes 'pm' (above), 'hs' (Hargreaves-Samani), 'thornthwaite' or 'none' (PET given with every member), and
 `routing=False` stops after ABCD: each member is then uploaded, run through PET -> ABCD and copied back on its own, and
 the run is bounded by the host -> device link.
+
+`run_parameter_ensemble` runs the other ensemble, parameter uncertainty: ONE forcing and many ABCD parameter tables.  The
+forcing is uploaded and its PET computed once; the tables go through ABCD several per launch (xan_abcd_run_sets reads
+each forcing value once for the sets of a thread), then through routing and the output reductions exactly as members.
 """
 
 from types import SimpleNamespace
@@ -57,6 +61,11 @@ STATS = ('mean', 'std', 'min', 'max')
 DROUGHT_VARS = ('q', 'soilmoisture')
 DROUGHT_SUMMARY = ('drought_months', 'events', 'longest_duration', 'peak_severity')
 DROUGHT_FIELDS = ('severity', 'intensity', 'duration')
+# Parameter tables per ABCD launch of an unrouted parameter ensemble (routed groups stay pairs, the routing launch's
+# unit).  B200, bench world (tools/parameter_ensemble_bench.py, DESIGN.md section 6): one xan_abcd_run_sets call takes
+# 0.38 ms per set at 4 sets and 0.34 at 8, against 0.53 per single-set call; 4 keeps most of the gain with half the
+# pinned output grids of 8 (3 x group per output variable).
+PARAMETER_SETS_PER_LAUNCH = 4
 
 
 def forcing_fields(pet):
@@ -207,6 +216,39 @@ class OutputSpec:
                 'quantiles={}{})'.format(self.output_in_year, self.output_unit, self.group_sums, self.member_fields,
                                          self.stats, self.ddof, self.quantiles,
                                          '' if self.drought is None else ', drought={!r}'.format(self.drought)))
+
+
+def parameter_sets(parameter_sets, n_rows):
+    """
+    ABCD parameter tables as float64 [P, n_rows, 5] (host only): `parameter_sets` is one [P, n_rows, 4 or 5] array or a
+    sequence of [n_rows, 4 or 5] tables (a, b, c, d[, m]; a 4-column table gets m = 0, no snow melt, as run_device
+    gives it).  Raises ValidationException for a table with another row count, another column count or another rank.
+    """
+    if hasattr(parameter_sets, 'ndim'):
+        a = np.asarray(parameter_sets, dtype=np.float64)
+        if a.ndim != 3:
+            raise C.ValidationException("parameter sets must be one [P, n_rows, 4 or 5] array or a sequence of "
+                                        "[n_rows, 4 or 5] tables, not an array of shape {}".format(a.shape))
+        tables = list(a)
+    else:
+        tables = [np.asarray(t, dtype=np.float64) for t in parameter_sets]
+    if not tables:
+        raise C.ValidationException("no parameter set given")
+    out = np.zeros((len(tables), int(n_rows), 5), dtype=np.float64)
+    for k, t in enumerate(tables):
+        if t.ndim != 2:
+            raise C.ValidationException("parameter set {} has shape {}, not [n_rows, 4 or 5]".format(k, t.shape))
+        if t.shape[0] != int(n_rows):
+            raise C.ValidationException("parameter set {} has {} rows, the statics' ABCD table {}".format(
+                k, t.shape[0], int(n_rows)))
+        if t.shape[1] not in (4, 5):
+            raise C.ValidationException("parameter set {} has {} columns, not 4 (a, b, c, d) or 5 (a, b, c, d, m)".format(
+                k, t.shape[1]))
+        out[k, :, :t.shape[1]] = t
+    return out
+
+
+_parameter_sets = parameter_sets      # run_parameter_ensemble's argument of the same name hides the function
 
 
 def merge_drought_counts(a, na, b, nb):
@@ -513,15 +555,19 @@ class EnsembleRunner:
             return th_mod.execute_device(fields['tair'], s.d_lat, s.start_yr)
         return fields['pet']
 
+    def _want(self):
+        """The ABCD outputs the back stage and the downloads read: q always, aet / sav when asked for or scanned."""
+        dvar = self._drought.var if self._drought is not None else None
+        return tuple(k for k, v in (('aet', 'aet'), ('q', 'q'), ('sav', 'soilmoisture'))
+                     if v in self.output_vars or k == 'q' or v == dvar)
+
     def _front(self, uploads):
         """Front stage, per member: wait for its upload, transposes, PET -> ABCD.  `uploads`: [(staged tensors, upload event)].
         Runs on the front stream (beside the routing launch of the group before); returns (PET Fields, ABCD results, event)."""
         s, torch = self.s, self._torch
         compute = torch.cuda.current_stream()
         stream = self.front if self.front is not None else compute
-        dvar = self._drought.var if self._drought is not None else None
-        want = tuple(k for k, v in (('aet', 'aet'), ('q', 'q'), ('sav', 'soilmoisture'))
-                     if v in self.output_vars or k == 'q' or v == dvar)
+        want = self._want()
         pets, ress = [], []
         with torch.cuda.stream(stream):
             while uploads:
@@ -540,6 +586,24 @@ class EnsembleRunner:
             ev = torch.cuda.Event()
             ev.record(stream)
         return pets, ress, ev
+
+    def _shared_forcing(self, forcing):
+        """The forcing of a parameter ensemble, uploaded, transposed and run through PET once (compute stream): (PET
+        Field, month-major forcing Fields)."""
+        staged, ev = self._upload(forcing, 0)
+        self._torch.cuda.current_stream().wait_event(ev)
+        fields = self._to_fields(staged)
+        return self._pet(fields), fields
+
+    def _front_sets(self, shared, pars):
+        """Front stage of a group of parameter sets (compute stream): ABCD of every table of `pars` [g, n_rows, 5] over
+        the shared forcing, one run_device_sets call; returns (PET Fields, ABCD results, event) like `_front`."""
+        s, (pet, fields) = self.s, shared
+        ress = abcd_mod.run_device_sets(s.plan, pars, pet, fields['precip'], fields['tmin'], s.nmonths, s.runoff_spinup,
+                                        want=self._want())
+        ev = self._torch.cuda.Event()
+        ev.record(self._torch.cuda.current_stream())
+        return [pet] * len(ress), ress, ev
 
     def _back(self, pets, ress):
         """One routing call for the group (with routing) and the basin aggregates per member (compute stream)."""
@@ -819,7 +883,7 @@ class EnsembleRunner:
         return {'members_in_drought': cnt, 'frequency': cnt / n, 'n_members': int(n)}
 
     # ---- driver ----------------------------------------------------------------------------------------------------------
-    def run(self, members):
+    def run(self, members, parameter_sets=None):
         """Generator: yields (index, {variable: host ndarray [ncell, nmonths], 'basin_aggregates': [n_agg_rows, nmonths,
         n_basins]}) in member order; the next members are being uploaded and a group of `group` members computed while
         the outputs of the group before are handed out.  With a spec the grids are [ncell, ntime] (none without member_fields), the
@@ -827,13 +891,22 @@ class EnsembleRunner:
         (`stats_partial` / `finalize_stats` once the generator is exhausted), its reduced fields kept on the device for
         the quantiles (`member_stack` / `finalize_quantiles`), and with spec.drought the result has 'drought':
         {'summary': {name: [ncell]}, 'thresholds'?: [nper, ncell], 'severity' / 'intensity' / 'duration'?:
-        [ncell, nmonths]} and the member is added to the drought counts (`drought_partial` / `finalize_drought`)."""
+        [ncell, nmonths]} and the member is added to the drought counts (`drought_partial` / `finalize_drought`).
+
+        With `parameter_sets` (float64 [P, n_rows, 5], see `parameter_sets`) `members` is ONE forcing dict, uploaded,
+        transposed and run through PET once before the loop, and item k is ABCD parameter table k over it: a group's
+        front stage is one run_device_sets call for its tables (pairs with routing, PARAMETER_SETS_PER_LAUNCH without)."""
         torch = self._torch
-        members = list(members)
-        if not members:
+        shared = None
+        if parameter_sets is None:
+            members = list(members)
+            n, g = len(members), self.group
+        else:
+            n, g = len(parameter_sets), (self.group if self.s.routing else PARAMETER_SETS_PER_LAUNCH)
+        if not n:
             return
         compute = torch.cuda.current_stream()
-        n, depth, g = len(members), self.prefetch_depth, self.group
+        depth = self.prefetch_depth
         # pinned output buffers in flight: the group being computed, the group before it on its way to the host, and the
         # results the caller still holds from the last hand-out - allocated before the pipeline starts, not inside it
         in_flight, grids = min(3 * g, n + g), {}          # cells x time steps -> pinned grids the pipeline holds
@@ -854,13 +927,18 @@ class EnsembleRunner:
         if self.spec is not None and self.spec.stats and self._stats_state is None:
             self._stats_state = {v: tuple(torch.empty((self.ntime, self.s.ld, 2), dtype=torch.float64, device='cuda')
                                           for _ in range(2)) for v in self.output_vars}
+        if parameter_sets is not None:
+            shared = self._shared_forcing(members)
+            d_sets = torch.from_numpy(np.ascontiguousarray(parameter_sets, dtype=np.float64)).cuda()
+            if self.timeline is not None:      # every set's entry starts at the one upload
+                self.timeline.extend(dict(self.timeline[-1]) for _ in range(n - 1))
         uploaded, next_up = {}, 0
         pending = []              # (index, host tensors, done event) of the members whose outputs are in flight
         computed = {}             # member -> completion event of its group's compute stage, to bound the uploads' run-ahead
 
         def pump(k):              # uploads of the members up to k + depth; member j waits for the compute of member j - depth - g
             nonlocal next_up
-            while next_up < n and next_up <= k + depth:
+            while shared is None and next_up < n and next_up <= k + depth:
                 old = next_up - depth - g
                 if old >= 0:
                     computed[old].synchronize()
@@ -870,6 +948,9 @@ class EnsembleRunner:
 
         def start_front(k0):      # front stage of the group starting at member k0
             ks = list(range(k0, min(n, k0 + g)))
+            if shared is not None:
+                fronts[k0] = self._front_sets(shared, d_sets[k0:ks[-1] + 1])
+                return
             if ks[-1] not in uploaded:
                 pump(ks[-1] - depth)
             fronts[k0] = self._front([uploaded.pop(k) for k in ks])
@@ -951,14 +1032,49 @@ def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=Tr
     (int32 [nmonths, ld], 278 MB at 67,420 cells x 1,032 months) and rank 0 adds the counts of the other ranks: integer
     sums are exact, so the counts and the frequency are bitwise the same for every number of ranks.
     """
+    members = list(members)
+    return _run_sharded(statics, len(members), lambda runner, mine: runner.run([members[i] for i in mine]),
+                        output_vars, aggregates, on_result, spec)
+
+
+def run_parameter_ensemble(statics, forcing, parameter_sets, output_vars=('q', 'avgchflow'), aggregates=True,
+                           on_result=None, spec=None):
+    """
+    A parameter ensemble: ABCD parameter table k (perturbations of a calibrated table, samples of a GLUE-style search)
+    over ONE forcing is "member k" of `run_ensemble`, and the return value has exactly its shape - per-set results,
+    'basin_aggregates' [P, rows, nmonths, n_basins], 'group_sums', 'ensemble_stats', 'ensemble_quantiles',
+    'drought_summary', 'ensemble_drought' and 'stats' (h2d_bytes, d2h_bytes, members_local).
+
+      forcing         one member dict with the keys of forcing_fields(statics.pet); it crosses the host -> device link
+                      and goes through PET once (once per rank under torch.distributed)
+      parameter_sets  one [P, n_rows, 4 or 5] array or a sequence of [n_rows, 4 or 5] tables (see `parameter_sets`);
+                      statics.abcd_pars is not run: it only fixes n_rows, the row count every table must have
+
+    Set k is bit-identical to the plug-in calls on table k (PET -> abcd_execute(..., pars_k, ...) -> mrtm.route) and
+    does not depend on the other sets.  ABCD runs several tables per launch (xan_abcd_run_sets); routing, the output
+    options and the across-set reductions are those of `run_ensemble`, and under torch.distributed the sets are dealt
+    to the ranks as members are.  'pet' is not an output: it is the same for every set.
+    """
+    if 'pet' in output_vars:
+        raise C.ValidationException("'pet' is not an output of a parameter ensemble: PET comes from the one forcing and "
+                                    "is the same for every parameter set (run_ensemble with the forcing returns it)")
+    missing = [k for k in forcing_fields(statics.pet) if k not in forcing]
+    if missing:
+        raise C.ValidationException("the forcing lacks {} (pet={!r})".format(missing, statics.pet))
+    sets = _parameter_sets(parameter_sets, statics.d_pars.shape[0])
+    return _run_sharded(statics, len(sets), lambda runner, mine: runner.run(forcing, parameter_sets=sets[mine]),
+                        output_vars, aggregates, on_result, spec)
+
+
+def _run_sharded(statics, n_members, run_local, output_vars, aggregates, on_result, spec):
+    """run_ensemble's driver over n_members items, this rank's share run by run_local(runner, indices)."""
     torch = C.torch_cuda()
     import torch.distributed as dist
-    members = list(members)
-    if spec is not None and spec.quantiles and len(members) > C.ENS_MAX_MEMBERS:
-        raise C.ValidationException("quantiles over {} members (at most {})".format(len(members), C.ENS_MAX_MEMBERS))
+    if spec is not None and spec.quantiles and n_members > C.ENS_MAX_MEMBERS:
+        raise C.ValidationException("quantiles over {} members (at most {})".format(n_members, C.ENS_MAX_MEMBERS))
     dist_on = dist.is_available() and dist.is_initialized()
     rank, world = (dist.get_rank(), dist.get_world_size()) if dist_on else (0, 1)
-    parts = sharding.partition_members(len(members), world)
+    parts = sharding.partition_members(n_members, world)
     mine = [int(i) for i in parts[rank]]
     runner = EnsembleRunner(statics, output_vars, aggregates, spec=spec)
     results = {}
@@ -968,7 +1084,7 @@ def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=Tr
                  for g in groups}
     drought = spec is not None and spec.drought is not None
     dr_local = torch.zeros((len(mine), len(DROUGHT_SUMMARY), statics.ncell), dtype=torch.float64) if drought else None
-    for j, res in runner.run([members[i] for i in mine]):
+    for j, res in run_local(runner, mine):
         if aggregates:
             agg_local[j] = torch.from_numpy(res['basin_aggregates'])
         for g in groups:
@@ -980,22 +1096,22 @@ def run_ensemble(statics, members, output_vars=('q', 'avgchflow'), aggregates=Tr
         else:
             results[mine[j]] = res
     if aggregates:      # every rank gets the basin aggregates of all members
-        results['basin_aggregates'] = sharding.gather_ragged_rows(mine, agg_local.cuda(), len(members)).cpu().numpy()
+        results['basin_aggregates'] = sharding.gather_ragged_rows(mine, agg_local.cuda(), n_members).cpu().numpy()
     if groups:
-        results['group_sums'] = {g: sharding.gather_ragged_rows(mine, grp_local[g].cuda(), len(members)).cpu().numpy()
+        results['group_sums'] = {g: sharding.gather_ragged_rows(mine, grp_local[g].cuda(), n_members).cpu().numpy()
                                  for g in groups}
     if drought:
-        results['drought_summary'] = sharding.gather_ragged_rows(mine, dr_local.cuda(), len(members)).cpu().numpy()
-    if drought and members:
+        results['drought_summary'] = sharding.gather_ragged_rows(mine, dr_local.cuda(), n_members).cpu().numpy()
+    if drought and n_members:
         partial = sharding.fold_to_rank0(runner.drought_partial(), [len(p) for p in parts], merge_drought_counts)
         if rank == 0:
-            results['ensemble_drought'] = runner.finalize_drought(partial, len(members))
-    if spec is not None and spec.stats and members:
+            results['ensemble_drought'] = runner.finalize_drought(partial, n_members)
+    if spec is not None and spec.stats and n_members:
         partial = sharding.fold_to_rank0(runner.stats_partial(), [len(p) for p in parts], runner.merge_stats)
         if rank == 0:
-            results['ensemble_stats'] = runner.finalize_stats(partial, len(members))
-            results['ensemble_stats']['n_members'] = len(members)
-    if spec is not None and spec.quantiles and members:
+            results['ensemble_stats'] = runner.finalize_stats(partial, n_members)
+            results['ensemble_stats']['n_members'] = n_members
+    if spec is not None and spec.quantiles and n_members:
         if world > 1:
             quant = runner.gather_quantiles([len(p) for p in parts])
         else:

@@ -69,6 +69,35 @@ def run_device(plan, pars, pet, precip, tmin, n_months, spinup_steps, want=('aet
     return out
 
 
+def run_device_sets(plan, pars_sets, pet, precip, tmin, n_months, spinup_steps, want=('aet', 'q', 'sav')):
+    """ABCD.emulate of every parameter table of `pars_sets` [P, n_rows, 4 or 5] over the same forcing: a list of P
+    `run_device` dicts, set k bit-identical to run_device(plan, pars_sets[k], ...).  One xan_abcd_run_sets call reads
+    the forcing once for up to C.ABCD_MAX_SETS tables; more tables take several calls."""
+    torch = C.torch_cuda()
+    e, p = C.as_field(pet), C.as_field(precip)
+    t = None if tmin is None else C.as_field(tmin)
+    n_months = int(n_months)
+    if e.nmonths < n_months or p.nmonths < n_months:
+        raise C.ValidationException("ABCD forcing shorter than n_months={}".format(n_months))
+    pr = pars_sets if isinstance(pars_sets, torch.Tensor) else torch.from_numpy(np.asarray(pars_sets, dtype=np.float64))
+    if pr.dim() != 3 or pr.shape[2] not in (4, 5):
+        raise C.ValidationException("parameter sets must be [P, n_rows, 4 or 5], not {}".format(tuple(pr.shape)))
+    pr = pr.to(device='cuda', dtype=torch.float64)
+    if pr.shape[2] == 4:   # no-snow parameter sets (a, b, c, d)
+        pr = torch.cat([pr, torch.zeros(pr.shape[:2] + (1,), dtype=pr.dtype, device=pr.device)], dim=2)
+    pr = pr.contiguous()
+    n_sets, n_rows = int(pr.shape[0]), int(pr.shape[1])
+    outs = [{k: C.Field.empty(e.ncell, n_months, e.ld) for k in want} for _ in range(n_sets)]
+    for s0 in range(0, n_sets, C.ABCD_MAX_SETS):
+        grp = outs[s0:s0 + C.ABCD_MAX_SETS]
+        ptrs = {k: (ctypes.c_void_p * len(grp))(*[o[k].t.data_ptr() for o in grp]) if k in want else None
+                for k in ('aet', 'q', 'sav')}
+        C.check(C.lib().xan_abcd_run_sets(plan._plan, len(grp), n_rows, C.ptr(e.t), C.ptr(p.t),
+                                          C.ptr(t.t if t is not None else None), C.ptr(pr[s0]), n_months,
+                                          int(spinup_steps), e.ld, ptrs['aet'], ptrs['q'], ptrs['sav'], C.stream_ptr()))
+    return outs
+
+
 def _basin_rows(n_basins, basin_ids, n_rows):
     """Row of the parameter table per cell, -1 for cells outside min_id .. min_id + n_basins - 1 (abcd.py:369-389)."""
     ids = np.asarray(basin_ids).astype(np.int64)
